@@ -96,6 +96,11 @@ EXTRAS = [
 ]
 
 
+# the reference's own filters (oracle/Makefile builds them from a HandBrake source tree); the CPU baseline runs them
+REF_SO = REPO / "oracle" / "_ref" / "libhbref.so"
+REF_HOWTO = "build it with `make -C oracle ref REF=<HandBrake source tree>`"
+
+
 class BenchStats(C.Structure):
     _fields_ = [("seconds", C.c_double), ("frames_out", C.c_int64), ("bytes_in", C.c_int64),
                 ("bytes_out", C.c_int64), ("checksum", C.c_uint64), ("ring_misses", C.c_int64)]
@@ -318,6 +323,38 @@ def plane_ptrs(t, dims, bps):
     return (C.c_void_p * 3)(*ptrs), (C.c_int * 3)(*strides)
 
 
+class _DeviceBytes:
+    """rows x pitch bytes of device memory, for torch.as_tensor"""
+
+    def __init__(self, ptr, pitch, rows):
+        self.__cuda_array_interface__ = {"shape": (rows, pitch), "typestr": "|u1", "data": (ptr, False), "version": 3}
+
+
+def device_plane(torch, ptr, pitch, w, h, bps):
+    """copy of an h x w plane (bps bytes a sample) at a device pointer with the given row pitch, as a numpy array"""
+    rows = torch.as_tensor(_DeviceBytes(ptr, pitch, h), device="cuda").cpu().numpy()
+    return np.ascontiguousarray(rows[:, : w * bps]).view(np.uint16 if bps == 2 else np.uint8)
+
+
+DUMP_BYTES = 63 * 10**6          # payload; the three .npy headers stay inside 64 MB
+
+
+def dump_outputs(out_dir, frames):
+    """frames: the output frames, each [Y, U, V] planes.  Writes y.npy, u.npy, v.npy as float32 of shape (frames, h, w)
+    when everything fits in DUMP_BYTES, else (frames, k) at the same k positions of every frame, k proportional to the
+    plane's size and drawn without replacement by np.random.default_rng(plane number), in raster order."""
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    total = len(frames) * sum(p.size for p in frames[0]) * 4
+    for i, name in enumerate(("y", "u", "v")):
+        a = np.stack([f[i] for f in frames]).astype(np.float32)
+        if total > DUMP_BYTES:
+            k = a[0].size * DUMP_BYTES // total
+            pos = np.sort(np.random.default_rng(i).choice(a[0].size, k, replace=False))
+            a = a.reshape(len(frames), -1)[:, pos]
+        np.save(out_dir / f"{name}.npy", a)
+
+
 def ncu_capture(workload, depth):
     """numbers of the committed `ncu --set full` capture of this workload's kernel (never measured live: a run under
     ncu is not a bench value)"""
@@ -355,9 +392,10 @@ class Ours:
         if rc != 0:
             raise RuntimeError(self.core.hbcu_last_error().decode())
 
-    def nlmeans_device_arm(self, wl, host, B, K, Wm, barrier=lambda: None, clock=None):
+    def nlmeans_device_arm(self, wl, host, B, K, Wm, barrier=lambda: None, clock=None, dump_dir=None):
         """kernel-only arm: one continuous stream whose raw frames are already in HBM.  Frame t+nf-1 is bordered
-        (upload_device) just before frame t is filtered, like the filter object does.  Returns (ms, kernel stats)."""
+        (upload_device) just before frame t is filtered, like the filter object does.  Returns (ms, kernel stats).
+        With dump_dir, the outputs of the last step still held in the handle's output slots are written there."""
         torch, core, ck = self.torch, self.core, self.ck
         W, H, depth, nf = wl["width"], wl["height"], wl["depth"], wl["nframes"]
         bps = 2 if depth > 8 else 1
@@ -366,19 +404,25 @@ class Ours:
         n_dev = max(8, min(32, int(420e6 // fb) + 1))                    # distinct device frames: > L2 (126 MB) in total
         dev = [torch.from_numpy(host[i % host.shape[0]]).cuda() for i in range(n_dev)]
         ptrs = [plane_ptrs(t, dims, bps) for t in dev]
-        cfg = nlm_config(self.flt, wl, self.gpu, ring=nf + 6, out_slots=4)
+        out_slots = 4
+        cfg = nlm_config(self.flt, wl, self.gpu, ring=nf + 6, out_slots=out_slots)
         h = C.c_void_p()
         ck(core.hbcu_nlmeans_create(C.byref(h), C.byref(cfg)))
         state = {"t": 0}
         for i in range(nf - 1):
             ck(core.hbcu_nlmeans_upload_device(h, C.c_int64(i), ptrs[i % n_dev][0], ptrs[i % n_dev][1]))
+        outp, outs = (C.c_void_p * 3)(), (C.c_int * 3)()
+        kept = {}           # frame -> (plane pointers, strides) of the step's last out_slots results, which no later frame overwrites
 
         def step():
             t0 = state["t"]
+            kept.clear()
             for t in range(t0, t0 + B):
                 u = t + nf - 1
                 ck(core.hbcu_nlmeans_upload_device(h, C.c_int64(u), ptrs[u % n_dev][0], ptrs[u % n_dev][1]))
-                ck(core.hbcu_nlmeans_filter_device(h, C.c_int64(t), nf, None, None))
+                ck(core.hbcu_nlmeans_filter_device(h, C.c_int64(t), nf, outp, outs))
+                if t >= t0 + B - out_slots:
+                    kept[t] = (list(outp), list(outs))
             state["t"] = t0 + B
 
         for _ in range(Wm):
@@ -399,6 +443,8 @@ class Ours:
         barrier()
         kms, kcalls = C.c_float(), C.c_int()
         ck(core.hbcu_nlmeans_kernel_ms(h, C.byref(kms), C.byref(kcalls)))
+        if dump_dir is not None:
+            dump_outputs(dump_dir, [[device_plane(torch, p, s, pw, ph, bps) for p, s, (pw, ph) in zip(*kept[t], dims)] for t in sorted(kept)])
         core.hbcu_nlmeans_destroy(h)
         del dev
         torch.cuda.empty_cache()
@@ -463,10 +509,9 @@ def reference_stream(names, settings, fmt, W, H, flags, host, chunk, budget_s, m
     """the unmodified reference filter(s) (oracle/_ref/libhbref.so) on the host cores: ONE continuous stream fed in
     chunks (a chunk = one full taskset cycle of the multithreaded filters) until the time budget is used; the serial
     EOF flush happens once, after the clock"""
-    so = REPO / "oracle" / "_ref" / "libhbref.so"
-    if not so.exists():
-        raise SystemExit("oracle/_ref/libhbref.so missing: run __graft_entry__.build() where /root/reference exists")
-    ref = C.CDLL(str(so))
+    if not REF_SO.exists():
+        raise SystemExit(f"{REF_SO} missing: {REF_HOWTO}")
+    ref = C.CDLL(str(REF_SO))
     bind_bench(ref)
     b = open_chain(ref, names, settings, fmt, W, H, flags)
     st = BenchStats()
@@ -699,7 +744,8 @@ def run_ours(args, wl, rank, world, local_rank):
 
     # ---------------- value: inputs resident in HBM ----------------
     clk = ClockSampler(gpu)
-    dev_ms_local, ks = ours.nlmeans_device_arm(wl, host, B, K, Wm, barrier=barrier, clock=clk)
+    dev_ms_local, ks = ours.nlmeans_device_arm(wl, host, B, K, Wm, barrier=barrier, clock=clk,
+                                               dump_dir=args.dump_outputs if rank == 0 else None)
     dev_ms = max_over_ranks(dev_ms_local)
     value = world * K * B / (dev_ms / 1e3)
 
@@ -787,14 +833,17 @@ def run_ours(args, wl, rank, world, local_rank):
     if plugin_multi is not None:
         out["plugin_multi_device"] = plugin_multi
     if world == 1 and not args.no_cpu_baseline:
-        _, out["cpu_baseline"] = cpu_baseline_nlmeans(wl, budget_s=12.0)
+        if REF_SO.exists():
+            _, out["cpu_baseline"] = cpu_baseline_nlmeans(wl, budget_s=12.0)
+        else:
+            out["cpu_baseline"] = {"value": None, "note": f"not measured: {REF_SO.relative_to(REPO)} is not built ({REF_HOWTO})"}
     if world == 1 and not args.no_extra:
         extra = []
         for ex in EXTRAS:
             if args.only_extra and args.only_extra not in ex["name"]:
                 continue
             try:
-                extra.append(run_extra(ours, ex, budget_cpu_s=8.0, with_cpu=not args.no_cpu_baseline))
+                extra.append(run_extra(ours, ex, budget_cpu_s=8.0, with_cpu=not args.no_cpu_baseline and REF_SO.exists()))
             except Exception as e:  # an extra must never take the headline line down with it
                 extra.append({"workload": ex["name"], "error": f"{type(e).__name__}: {e}"})
         out["extra"] = extra
@@ -887,6 +936,9 @@ def main():
     ap.add_argument("--plugin-warm", type=int, default=256, help=argparse.SUPPRESS)
     ap.add_argument("--block", type=int, default=8, help="frames per device turn of the plugin's multi-device dealing")
     ap.add_argument("--inflight", type=int, default=6, help="frames in flight in the e2e arm (the filter's `threads` setting)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the Y/U/V output planes of the last step's final frames (the frames the "
+                         "kernel-only arm still holds) to DIR/{y,u,v}.npy as float32; a fixed sample of positions when larger than 64 MB")
     args = ap.parse_args()
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3                     # timing rule: at least three warm-up steps

@@ -28,11 +28,19 @@ def _have_gpu():
 
 @pytest.fixture(scope="session")
 def ref():
-    """the reference's own filters (oracle/_ref/libhbref.so), built from /root/reference when present"""
+    """the reference's own filters: their stored runs (tests/reference_runs.py); with HBCU_RECORD_REFERENCE=<file> the
+    calls run on oracle/_ref/libhbref.so and the stored runs plus every call made are written to <file>"""
+    from reference_runs import ReferenceRuns
+    out = os.environ.get("HBCU_RECORD_REFERENCE")
+    if not out:
+        yield ReferenceRuns.load()
+        return
     from handbrake_b200.hblib import FilterLib
     if not REF_SO.exists():
-        pytest.skip("oracle/_ref/libhbref.so not built (needs /root/reference at build time)")
-    return FilterLib(REF_SO)
+        pytest.fail("HBCU_RECORD_REFERENCE is set but oracle/_ref/libhbref.so is not built")
+    runs = ReferenceRuns.load(FilterLib(REF_SO))
+    yield runs
+    runs.save(out)
 
 
 @pytest.fixture(scope="session")

@@ -60,7 +60,7 @@ def test_templates_match_reference(ref):
                  ("hb_filter_decomb_cuda", "hb_filter_decomb"), ("hb_filter_lapsharp_cuda", "hb_filter_lapsharp"),
                  ("hb_filter_unsharp_cuda", "hb_filter_unsharp"), ("hb_filter_chroma_smooth_cuda", "hb_filter_chroma_smooth"),
                  ("hb_filter_denoise_cuda", "hb_filter_denoise"), ("hb_filter_detelecine_cuda", "hb_filter_detelecine")):
-        assert Head.in_dll(flt.lib, a).settings_template == Head.in_dll(ref.lib, b).settings_template, a
+        assert Head.in_dll(flt.lib, a).settings_template == ref.settings_template(b), a
 
 
 def test_no_cpu_fallback_without_gpu():
@@ -102,19 +102,3 @@ def test_product_filter_library_carries_no_libhb_stand_in():
     sh = subprocess.run(["nm", "-D", str(shim)], capture_output=True, text=True).stdout
     assert " T hb_harness_run_chain" in sh and " T hb_bench_stream" in sh and " T hb_buffer_init" in sh
     assert "hbcu_" not in "\n".join(l for l in sh.splitlines() if " U " in l)      # the stand-in knows nothing of the product
-
-
-def test_filter_sources_compile_against_the_real_libhb_headers():
-    """INTEGRATION.md claims the *_cuda.c sources drop into a HandBrake tree unchanged: syntax-only compile against the
-    reference's own handbrake/*.h (tools/check_real_headers.sh; libav/jansson are type-only stubs).  The only names the
-    real tree lacks are the integration patch itself: HBCU_DEVICE and the three fifo.c hooks."""
-    import subprocess
-    ref = Path("/root/reference/libhb")
-    if not (ref / "handbrake" / "internal.h").exists():
-        pytest.skip("no reference tree on this machine")
-    r = subprocess.run(["bash", str(REPO / "tools" / "check_real_headers.sh"), str(ref)], capture_output=True, text=True)
-    assert r.returncode == 0, r.stdout + r.stderr
-    lines = [l for l in r.stdout.splitlines() if ": errors=" in l]
-    assert len(lines) >= 10 and all("errors=0 other_warnings=0" in l for l in lines), r.stdout
-    hooks = set(re.findall(r"'(hb_shim_[a-z_]+)'", r.stdout))
-    assert hooks == {"hb_shim_set_frame_allocator", "hb_shim_set_device_release", "hb_shim_set_device_retain"}

@@ -3,6 +3,7 @@ import numpy as np
 import pytest
 
 from handbrake_b200 import synth
+from reference_runs import differing_frames
 from test_oracle import DECOMB_CASES, decomb_inputs
 
 pytestmark = pytest.mark.gpu
@@ -18,8 +19,7 @@ def compare(ref, cuda, s, clip, fmt, w, h, flags, combed):
     assert np.array_equal(g.flags, r.flags) and np.array_equal(g.combed, r.combed)
     assert g.vrate == r.vrate
     if not np.array_equal(g.frames, r.frames):
-        d = g.frames != r.frames
-        raise AssertionError(f"{s}: {np.count_nonzero(d)} bytes differ in frames {np.argwhere(d.any(axis=1)).ravel()[:8]}")
+        raise AssertionError(f"{s}: frames {differing_frames(g.frames, r.frames)[:8]} differ")
 
 
 @pytest.mark.parametrize("mode,parity,tags", DECOMB_CASES)

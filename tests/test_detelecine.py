@@ -2,13 +2,14 @@
 
 oracle/_ref/libhostlogic.so is the PRODUCT's host-side state machine (handbrake_b200/libhb/detelecine_cuda.c,
 compiled untouched) with its device calls redirected to the plain-C restatement oracle/port/detelecine_port.c.  Pinned
-here, frame for frame, against the reference's own hb_filter_detelecine compiled from /root/reference.  On the GPU box the
-same host code drives the CUDA kernels and tests/test_detelecine_gpu.py compares that with the reference."""
+here, frame for frame, against the stored runs of the reference's own hb_filter_detelecine (tests/reference_runs.py).  On
+the GPU box the same host code drives the CUDA kernels and tests/test_detelecine_gpu.py compares that with the reference."""
 import numpy as np
 import pytest
 
 from handbrake_b200 import synth
 from conftest import ORACLE_DIR
+from reference_runs import differing_frames
 
 FMT = {8: synth.PIX_FMT_YUV420P, 10: synth.PIX_FMT_YUV420P10}
 HOSTLOGIC_SO = ORACLE_DIR / "_ref" / "libhostlogic.so"      # see tests/test_hostlogic.py
@@ -43,8 +44,7 @@ def compare(r, g):
     assert g.frames.shape == r.frames.shape, (g.frames.shape, r.frames.shape)
     assert np.array_equal(g.start, r.start) and np.array_equal(g.stop, r.stop) and np.array_equal(g.flags, r.flags)
     if not np.array_equal(g.frames, r.frames):
-        d = g.frames != r.frames
-        raise AssertionError(f"{np.count_nonzero(d)} bytes differ in frames {np.argwhere(d.any(axis=1)).ravel()[:8]}")
+        raise AssertionError(f"frames {differing_frames(g.frames, r.frames)[:8]} differ")
 
 
 @pytest.mark.parametrize("kw,settings", DETELECINE_CASES)

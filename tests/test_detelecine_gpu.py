@@ -1,5 +1,5 @@
 """GPU parity: hb_filter_detelecine_cuda (host state machine + CUDA metrics / reductions / field weaving) against the
-reference's hb_filter_detelecine compiled from /root/reference -- pictures, timestamps, flags, which frames are dropped."""
+reference's hb_filter_detelecine (its stored runs, tests/reference_runs.py) -- pictures, timestamps, flags, which frames are dropped."""
 import numpy as np
 import pytest
 

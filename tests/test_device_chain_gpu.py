@@ -7,6 +7,7 @@ import numpy as np
 import pytest
 
 from handbrake_b200 import LIBHBCU, synth
+from reference_runs import differing_frames
 from test_oracle import decomb_inputs
 
 pytestmark = pytest.mark.gpu
@@ -26,8 +27,7 @@ def same(r, g):
     assert g.frames.shape == r.frames.shape, (g.frames.shape, r.frames.shape)
     assert np.array_equal(g.start, r.start)
     if not np.array_equal(g.frames, r.frames):
-        d = g.frames != r.frames
-        raise AssertionError(f"{np.count_nonzero(d)} bytes differ in frames {np.argwhere(d.any(axis=1)).ravel()[:8]}")
+        raise AssertionError(f"frames {differing_frames(g.frames, r.frames)[:8]} differ")
 
 
 @pytest.mark.parametrize("depth,w,h", [(8, 333, 211), (10, 330, 210), (8, 640, 360)])

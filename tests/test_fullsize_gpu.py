@@ -4,6 +4,7 @@ import numpy as np
 import pytest
 
 from handbrake_b200 import synth
+from reference_runs import differing_frames
 from test_oracle import decomb_inputs
 
 pytestmark = pytest.mark.gpu
@@ -13,8 +14,7 @@ FMT = {8: synth.PIX_FMT_YUV420P, 10: synth.PIX_FMT_YUV420P10}
 def same(r, g):
     assert g.frames.shape == r.frames.shape
     if not np.array_equal(g.frames, r.frames):
-        d = g.frames != r.frames
-        raise AssertionError(f"{np.count_nonzero(d)} bytes differ in frames {np.argwhere(d.any(axis=1)).ravel()[:8]}")
+        raise AssertionError(f"frames {differing_frames(g.frames, r.frames)[:8]} differ")
     assert np.array_equal(g.start, r.start) and list(g.combed) == list(r.combed)
 
 

@@ -2,8 +2,9 @@
 tables, look-ahead buffering, EOF flush, output order and properties).
 
 oracle/_ref/libhostlogic.so is handbrake_b200/libhb/*_cuda.c compiled UNTOUCHED, with every hbcu_* device call renamed to
-a plain-C stand-in built on the restatement (oracle/port/hostlogic_*.c).  Compared here with the reference's own filter
-objects compiled from /root/reference.  On the GPU box the same host code drives the CUDA kernels (tests/test_*_gpu.py)."""
+a plain-C stand-in built on the restatement (oracle/port/hostlogic_*.c).  Compared here with the stored runs of the
+reference's own filter objects (tests/reference_runs.py).  On the GPU box the same host code drives the CUDA kernels
+(tests/test_*_gpu.py)."""
 import ctypes as C
 import hashlib
 import json
@@ -14,6 +15,7 @@ import pytest
 
 from handbrake_b200 import synth
 from conftest import ORACLE_DIR
+from reference_runs import differing_frames
 
 FMT = {8: synth.PIX_FMT_YUV420P, 10: synth.PIX_FMT_YUV420P10}
 HOSTLOGIC_SO = ORACLE_DIR / "_ref" / "libhostlogic.so"
@@ -32,8 +34,7 @@ def same_stream(r, g):
     assert g.frames.shape == r.frames.shape, (g.frames.shape, r.frames.shape)
     assert np.array_equal(g.start, r.start) and np.array_equal(g.stop, r.stop) and np.array_equal(g.flags, r.flags)
     if not np.array_equal(g.frames, r.frames):
-        d = g.frames != r.frames
-        raise AssertionError(f"{np.count_nonzero(d)} bytes differ in frames {np.argwhere(d.any(axis=1)).ravel()[:8]}")
+        raise AssertionError(f"frames {differing_frames(g.frames, r.frames)[:8]} differ")
 
 
 NLMEANS_SETTINGS = [

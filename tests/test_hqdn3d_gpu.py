@@ -3,6 +3,7 @@ import numpy as np
 import pytest
 
 from handbrake_b200 import synth
+from reference_runs import differing_frames
 from test_oracle import HQDN3D_CASES
 
 pytestmark = pytest.mark.gpu
@@ -16,8 +17,7 @@ def same(r, g):
     assert g.frames.shape == r.frames.shape
     assert np.array_equal(g.start, r.start)
     if not np.array_equal(g.frames, r.frames):
-        d = np.abs(g.frames.astype(np.int32) - r.frames.astype(np.int32))
-        raise AssertionError(f"max abs {d.max()}, {np.count_nonzero(d)} bytes differ, frames {np.argwhere(d.max(axis=1) > 0).ravel()[:8]}")
+        raise AssertionError(f"frames {differing_frames(g.frames, r.frames)[:8]} differ")
 
 
 @pytest.mark.parametrize("settings", [c[0] for c in HQDN3D_CASES])

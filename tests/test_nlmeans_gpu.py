@@ -3,6 +3,7 @@ import numpy as np
 import pytest
 
 from handbrake_b200 import synth
+from reference_runs import differing_frames
 
 pytestmark = pytest.mark.gpu
 
@@ -20,9 +21,7 @@ def assert_same(r, g):
     assert g.frames.shape == r.frames.shape
     assert np.array_equal(g.start, r.start)
     if not np.array_equal(g.frames, r.frames):
-        d = np.abs(g.frames.astype(np.int32) - r.frames.astype(np.int32))
-        bad = np.argwhere(d.max(axis=1) > 0).ravel()
-        raise AssertionError(f"mismatch: max abs {d.max()}, {np.count_nonzero(d)} bytes differ, frames {bad[:8]}")
+        raise AssertionError(f"mismatch: frames {differing_frames(g.frames, r.frames)[:8]} differ")
 
 
 @pytest.mark.parametrize("strength", [3, 6, 10])

@@ -10,6 +10,7 @@ import pytest
 
 import handbrake_b200
 from handbrake_b200 import synth
+from reference_runs import differing_frames
 
 pytestmark = pytest.mark.gpu
 
@@ -25,8 +26,7 @@ def same(a, b):
     assert a.frames.shape == b.frames.shape
     assert np.array_equal(a.start, b.start) and np.array_equal(a.stop, b.stop)
     if not np.array_equal(a.frames, b.frames):
-        d = a.frames != b.frames
-        raise AssertionError(f"{np.count_nonzero(d)} bytes differ in frames {np.argwhere(d.any(axis=1)).ravel()[:8]}")
+        raise AssertionError(f"frames {differing_frames(a.frames, b.frames)[:8]} differ")
 
 
 CASES = [

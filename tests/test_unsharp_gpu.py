@@ -4,6 +4,7 @@ import numpy as np
 import pytest
 
 from handbrake_b200 import synth
+from reference_runs import differing_frames
 from test_oracle import UNSHARP_CASES, CHROMA_SMOOTH_CASES
 
 pytestmark = pytest.mark.gpu
@@ -17,8 +18,7 @@ def same(r, g):
     assert g.frames.shape == r.frames.shape
     assert np.array_equal(g.start, r.start)
     if not np.array_equal(g.frames, r.frames):
-        d = np.abs(g.frames.astype(np.int32) - r.frames.astype(np.int32))
-        raise AssertionError(f"max abs {d.max()}, {np.count_nonzero(d)} bytes differ, frames {np.argwhere(d.max(axis=1) > 0).ravel()[:8]}")
+        raise AssertionError(f"frames {differing_frames(g.frames, r.frames)[:8]} differ")
 
 
 @pytest.mark.parametrize("settings", [c[0] for c in UNSHARP_CASES])
