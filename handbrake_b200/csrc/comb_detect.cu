@@ -6,14 +6,14 @@
 //   check_filtered_combing_mask / check_combing_mask      comb_detect.c:221-276, 384-454
 //   check_combing_results                                 comb_detect.c:1029-1049
 // The reference runs five fork/join tasksets over row segments; here one frame is
-// three kernels on one stream:
-//   comb_mask_kernel    raw mask from the prev/cur/next luma planes (gamma values come from the
-//                       host-built table staged in shared memory, so the float results are the
-//                       reference's bit for bit; no FMA contraction: -fmad=false + explicit rn ops)
-//   comb_filter_kernel  filter -> erode -> dilate -> erode fused in shared memory (4-pixel halo),
-//                       intermediate masks never touch HBM
-//   comb_score_kernel   block sums -> LIGHT/HEAVY flags (atomicOr), verdict read back through
-//                       pinned memory
+// three kernels on one stream, all on a one-bit-per-pixel mask:
+//   comb_mask_bits2_kernel   raw mask from the prev/cur/next luma planes (gamma values come from the
+//                            host-built table staged in shared memory, so the float results are the
+//                            reference's bit for bit; no FMA contraction: -fmad=false + explicit rn ops)
+//   comb_filter_bits_kernel  filter -> erode -> dilate -> erode fused in shared memory,
+//                            intermediate masks never touch HBM
+//   comb_score_bits_kernel   block sums -> LIGHT/HEAVY flags (atomicOr), verdict read back through
+//                            pinned memory
 // Integer work is bit-exact by construction; the segment decomposition of the reference does
 // not influence its result (block grid is globally aligned, SURVEY.md 8a/a14).
 #include "hbcu_common.h"
@@ -43,207 +43,7 @@ struct CombParams
 };
 
 // ---------------------------------------------------------------------------
-// raw mask: one thread per pixel, rows [2, h-2); everything else is 0
-// ---------------------------------------------------------------------------
-template <typename PIX, bool GAMMA>
-__global__ void __launch_bounds__(256) comb_mask_kernel(const PIX *__restrict__ prev, const PIX *__restrict__ cur,
-                                                       const PIX *__restrict__ next, uint8_t *__restrict__ mask,
-                                                       int mpitch, CombParams p)
-{
-    extern __shared__ float s_lut[];
-    if (GAMMA)
-    {
-        for (int i = threadIdx.y * blockDim.x + threadIdx.x; i < p.lut_size; i += blockDim.x * blockDim.y)
-            s_lut[i] = p.gamma_lut[i];
-        __syncthreads();
-    }
-    const int x = blockIdx.x * blockDim.x + threadIdx.x;
-    const int y = blockIdx.y * blockDim.y + threadIdx.y;
-    if (x >= p.w || y >= p.h) return;
-    uint8_t m = 0;
-    if (y >= 2 && y < p.h - 2)
-    {
-        const size_t i = (size_t)y * p.pitch + x;
-        const int pc = cur[i], pu1 = cur[i - p.pitch], pd1 = cur[i + p.pitch];
-        if (GAMMA)
-        {
-            const float gc = s_lut[pc], gu1 = s_lut[pu1], gd1 = s_lut[pd1];
-            const float up = __fsub_rn(gc, gu1), down = __fsub_rn(gc, gd1);
-            if ((up > p.g_athresh && down > p.g_athresh) || (up < -p.g_athresh && down < -p.g_athresh))
-            {
-                int motion = 0;
-                if (p.g_mthresh > 0)
-                {
-                    const float qc = s_lut[prev[i]], nc = s_lut[next[i]];
-                    const float qu1 = s_lut[prev[i - p.pitch]], qd1 = s_lut[prev[i + p.pitch]];
-                    const float nu1 = s_lut[next[i - p.pitch]], nd1 = s_lut[next[i + p.pitch]];
-                    if (fabsf(__fsub_rn(qc, gc)) > p.g_mthresh && fabsf(__fsub_rn(gu1, nu1)) > p.g_mthresh &&
-                        fabsf(__fsub_rn(gd1, nd1)) > p.g_mthresh)
-                        motion++;
-                    if (fabsf(__fsub_rn(nc, gc)) > p.g_mthresh && fabsf(__fsub_rn(qu1, gu1)) > p.g_mthresh &&
-                        fabsf(__fsub_rn(qd1, gd1)) > p.g_mthresh)
-                        motion++;
-                }
-                else
-                    motion = 1;
-                if (motion || p.force)
-                {
-                    const float gu2 = s_lut[cur[i - 2 * p.pitch]], gd2 = s_lut[cur[i + 2 * p.pitch]];
-                    // fabs(up2 + 4*c + down2 - 3*(up1 + down1)), left to right, no contraction
-                    const float lhs = __fadd_rn(__fadd_rn(gu2, __fmul_rn(4.0f, gc)), gd2);
-                    const float rhs = __fmul_rn(3.0f, __fadd_rn(gu1, gd1));
-                    if (fabsf(__fsub_rn(lhs, rhs)) > p.g_athresh6) m = 1;
-                }
-            }
-        }
-        else
-        {
-            const int up = pc - pu1, down = pc - pd1;
-            if ((up > p.athresh && down > p.athresh) || (up < -p.athresh && down < -p.athresh))
-            {
-                int motion = 0;
-                if (p.mthresh > 0)
-                {
-                    const int qc = prev[i], nc = next[i];
-                    const int qu1 = prev[i - p.pitch], qd1 = prev[i + p.pitch];
-                    const int nu1 = next[i - p.pitch], nd1 = next[i + p.pitch];
-                    if (abs(qc - pc) > p.mthresh && abs(pu1 - nu1) > p.mthresh && abs(pd1 - nd1) > p.mthresh) motion++;
-                    if (abs(nc - pc) > p.mthresh && abs(qu1 - pu1) > p.mthresh && abs(qd1 - pd1) > p.mthresh) motion++;
-                }
-                else
-                    motion = 1;
-                if (motion || p.force)
-                {
-                    const int pu2 = cur[i - 2 * p.pitch], pd2 = cur[i + 2 * p.pitch];
-                    if (p.spatial_metric == 0)
-                        m = (abs(pc - pd2) < p.c32min) && (abs(pc - pd1) > p.c32max);
-                    else if (p.spatial_metric == 1)
-                        m = (pu1 - pc) * (pd1 - pc) > p.athresh_sq;
-                    else if (p.spatial_metric == 2)
-                        m = abs(pu2 + 4 * pc + pd2 - 3 * (pu1 + pd1)) > p.athresh6;
-                }
-            }
-        }
-    }
-    mask[(size_t)y * mpitch + x] = m;
-}
-
-// ---------------------------------------------------------------------------
-// mask filter chain fused in shared memory.  Output tile FT_W x FT_H, halo 4.
-// Every intermediate mask is 0 outside [1,w-2] x [1,h-2] (the reference never writes there).
-// ---------------------------------------------------------------------------
-constexpr int FT_W = 64, FT_H = 32, FT_HALO = 4;
-constexpr int FS_W = FT_W + 2 * FT_HALO, FS_H = FT_H + 2 * FT_HALO;
-
-enum { OP_CLASSIC = 0, OP_HV = 1, OP_ERODE = 2, OP_DILATE = 3 };
-
-__device__ __forceinline__ void filter_stage(const uint8_t *src, uint8_t *dst, int op, int shrink,
-                                             int gx0, int gy0, int w, int h)
-{
-    // computes dst on the tile region shrunk by `shrink` pixels per side from src (valid one pixel wider)
-    const int rw = FS_W - 2 * shrink, rh = FS_H - 2 * shrink;
-    for (int i = threadIdx.x; i < rw * rh; i += blockDim.x)
-    {
-        const int lx = shrink + i % rw, ly = shrink + i / rw;
-        const int gx = gx0 + lx, gy = gy0 + ly;
-        uint8_t v = 0;
-        if (gx >= 1 && gx <= w - 2 && gy >= 1 && gy <= h - 2)
-        {
-            const uint8_t *s = src + ly * FS_W + lx;
-            if (op == OP_CLASSIC || op == OP_HV)
-            {
-                const int hc = s[-1] & s[0] & s[1];
-                const int vc = s[-FS_W] & s[0] & s[FS_W];
-                v = op == OP_CLASSIC ? hc : (hc & vc);
-            }
-            else
-            {
-                const int count = s[-FS_W - 1] + s[-FS_W] + s[-FS_W + 1] + s[-1] + s[1] + s[FS_W - 1] + s[FS_W] + s[FS_W + 1];
-                if (op == OP_ERODE) v = s[0] ? (count >= 2) : 0;
-                else                v = s[0] ? 1 : (count >= 4);
-            }
-        }
-        dst[ly * FS_W + lx] = v;
-    }
-    __syncthreads();
-}
-
-__global__ void __launch_bounds__(256) comb_filter_kernel(const uint8_t *__restrict__ mask, uint8_t *__restrict__ out,
-                                                         int mpitch, int w, int h, int filter_mode)
-{
-    __shared__ uint8_t a[FS_W * FS_H], b[FS_W * FS_H];
-    const int gx0 = blockIdx.x * FT_W - FT_HALO, gy0 = blockIdx.y * FT_H - FT_HALO;
-    for (int i = threadIdx.x; i < FS_W * FS_H; i += blockDim.x)
-    {
-        const int gx = gx0 + i % FS_W, gy = gy0 + i / FS_W;
-        a[i] = (gx >= 0 && gx < w && gy >= 0 && gy < h) ? mask[(size_t)gy * mpitch + gx] : 0;
-        b[i] = 0;
-    }
-    __syncthreads();
-    const uint8_t *res;
-    if (filter_mode == 1)
-    {
-        filter_stage(a, b, OP_CLASSIC, 1, gx0, gy0, w, h);
-        res = b;
-    }
-    else
-    {
-        filter_stage(a, b, OP_HV, 1, gx0, gy0, w, h);          // mask -> temp
-        if (filter_mode == 2)
-        {
-            filter_stage(b, a, OP_ERODE, 2, gx0, gy0, w, h);   // temp -> filtered
-            filter_stage(a, b, OP_DILATE, 3, gx0, gy0, w, h);  // filtered -> temp
-            filter_stage(b, a, OP_ERODE, 4, gx0, gy0, w, h);   // temp -> filtered
-            res = a;
-        }
-        else
-        {
-            res = nullptr;                                      // nothing ever writes mask_filtered: stays 0
-        }
-    }
-    for (int i = threadIdx.x; i < FT_W * FT_H; i += blockDim.x)
-    {
-        const int lx = FT_HALO + i % FT_W, ly = FT_HALO + i / FT_W;
-        const int gx = gx0 + lx, gy = gy0 + ly;
-        if (gx < w && gy < h) out[(size_t)gy * mpitch + gx] = res ? res[ly * FS_W + lx] : 0;
-    }
-}
-
-// ---------------------------------------------------------------------------
-// block scores -> flags: bit0 some block >= threshold/2, bit1 some block > threshold
-// one warp per block
-// ---------------------------------------------------------------------------
-__global__ void __launch_bounds__(128) comb_score_kernel(const uint8_t *__restrict__ m, int mpitch, int w, int h,
-                                                        int bw, int bh, int nbx, int nby, int threshold, int filtered,
-                                                        int *__restrict__ flags)
-{
-    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
-    if (warp >= nbx * nby) return;
-    const int x0 = (warp % nbx) * bw, y0 = (warp / nbx) * bh;
-    int score = 0;
-    for (int i = lane; i < bw * bh; i += 32)
-    {
-        const int x = x0 + i % bw, y = y0 + i / bw;
-        const uint8_t *p = m + (size_t)y * mpitch + x;
-        if (filtered) score += p[0];
-        else if (x == 0) score += p[0] & p[1];
-        else if (x == w - 1) score += p[-1] & p[0];
-        else score += p[-1] & p[0] & p[1];
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) score += __shfl_xor_sync(0xffffffffu, score, o);
-    if (lane == 0)
-    {
-        int f = 0;
-        if (score >= threshold / 2) f |= 1;
-        if (score > threshold) f |= 2;
-        if (f) atomicOr(flags, f);
-    }
-}
-
-
-// ---------------------------------------------------------------------------
-// Bit-packed path (default).  The combing mask is one bit per pixel: a warp evaluates 32 neighbouring pixels and
+// The combing mask is one bit per pixel: a warp evaluates 32 neighbouring pixels and
 // __ballot_sync() delivers their mask word; the whole filter chain (filter -> erode -> dilate -> erode, comb_detect.c:
 // 556-966) then runs on 32 pixels per integer instruction -- neighbours are shifted words, the "n of 8 neighbours"
 // rules a bit-sliced adder tree -- and block scores are popcounts.  Mask traffic drops from 8 bytes to 4 bits per pixel
@@ -254,97 +54,7 @@ __global__ void __launch_bounds__(128) comb_score_kernel(const uint8_t *__restri
 constexpr int kGuard = 4;
 constexpr int kMaskRows = 16;                  // rows a thread marches down in the mask kernel
 
-template <typename PIX, bool GAMMA>
-__device__ __forceinline__ int comb_px(const PIX *__restrict__ prev, const PIX *__restrict__ next, const float *__restrict__ lut,
-                                       const CombParams &p, size_t i, int pu2, int pu1, int pc, int pd1, int pd2,
-                                       float gu2, float gu1, float gc, float gd1, float gd2)
-{
-    if (GAMMA)
-    {
-        const float up = __fsub_rn(gc, gu1), down = __fsub_rn(gc, gd1);
-        if (!((up > p.g_athresh && down > p.g_athresh) || (up < -p.g_athresh && down < -p.g_athresh))) return 0;
-        int motion = 0;
-        if (p.g_mthresh > 0)
-        {
-            const float qc = lut[prev[i]], nc = lut[next[i]];
-            const float qu1 = lut[prev[i - p.pitch]], qd1 = lut[prev[i + p.pitch]];
-            const float nu1 = lut[next[i - p.pitch]], nd1 = lut[next[i + p.pitch]];
-            if (fabsf(__fsub_rn(qc, gc)) > p.g_mthresh && fabsf(__fsub_rn(gu1, nu1)) > p.g_mthresh &&
-                fabsf(__fsub_rn(gd1, nd1)) > p.g_mthresh)
-                motion++;
-            if (fabsf(__fsub_rn(nc, gc)) > p.g_mthresh && fabsf(__fsub_rn(qu1, gu1)) > p.g_mthresh &&
-                fabsf(__fsub_rn(qd1, gd1)) > p.g_mthresh)
-                motion++;
-        }
-        else
-            motion = 1;
-        if (!(motion || p.force)) return 0;
-        const float lhs = __fadd_rn(__fadd_rn(gu2, __fmul_rn(4.0f, gc)), gd2);     // left to right, no contraction
-        const float rhs = __fmul_rn(3.0f, __fadd_rn(gu1, gd1));
-        return fabsf(__fsub_rn(lhs, rhs)) > p.g_athresh6;
-    }
-    const int up = pc - pu1, down = pc - pd1;
-    if (!((up > p.athresh && down > p.athresh) || (up < -p.athresh && down < -p.athresh))) return 0;
-    int motion = 0;
-    if (p.mthresh > 0)
-    {
-        const int qc = prev[i], nc = next[i];
-        const int qu1 = prev[i - p.pitch], qd1 = prev[i + p.pitch];
-        const int nu1 = next[i - p.pitch], nd1 = next[i + p.pitch];
-        if (abs(qc - pc) > p.mthresh && abs(pu1 - nu1) > p.mthresh && abs(pd1 - nd1) > p.mthresh) motion++;
-        if (abs(nc - pc) > p.mthresh && abs(qu1 - pu1) > p.mthresh && abs(qd1 - pd1) > p.mthresh) motion++;
-    }
-    else
-        motion = 1;
-    if (!(motion || p.force)) return 0;
-    if (p.spatial_metric == 0) return (abs(pc - pd2) < p.c32min) && (abs(pc - pd1) > p.c32max);
-    if (p.spatial_metric == 1) return (pu1 - pc) * (pd1 - pc) > p.athresh_sq;
-    if (p.spatial_metric == 2) return abs(pu2 + 4 * pc + pd2 - 3 * (pu1 + pd1)) > p.athresh6;
-    return 0;
-}
-
-// one warp = 32 neighbouring columns marching down kMaskRows rows: every luma sample of the current frame is read
-// once (five-row window in registers); previous / next frame only where the spatial test already fired
-template <typename PIX, bool GAMMA>
-__global__ void __launch_bounds__(256) comb_mask_bits_kernel(const PIX *__restrict__ prev, const PIX *__restrict__ cur,
-                                                            const PIX *__restrict__ next, uint32_t *__restrict__ bits,
-                                                            int wpitch, CombParams p)
-{
-    extern __shared__ float s_lut[];
-    if (GAMMA)
-    {
-        for (int i = threadIdx.x; i < p.lut_size; i += blockDim.x) s_lut[i] = p.gamma_lut[i];
-        __syncthreads();
-    }
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int wx = blockIdx.x * 8 + warp;
-    if (wx * 32 >= p.w) return;                               // whole warp
-    const int x = wx * 32 + lane;
-    const bool colok = x < p.w;
-    const int xc = colok ? x : p.w - 1;
-    const int y0 = blockIdx.y * kMaskRows;
-    // the whole column segment first (kMaskRows + 4 independent loads in flight), its gamma values looked up once
-    int c[kMaskRows + 4];
-    float g[kMaskRows + 4];
-#pragma unroll
-    for (int k = 0; k < kMaskRows + 4; k++)
-        c[k] = cur[(size_t)min(max(y0 - 2 + k, 0), p.h - 1) * p.pitch + xc];
-#pragma unroll
-    for (int k = 0; k < kMaskRows + 4; k++)
-        g[k] = GAMMA ? s_lut[c[k]] : 0.f;
-#pragma unroll
-    for (int r = 0; r < kMaskRows; r++)
-    {
-        const int y = y0 + r;
-        if (y >= p.h) break;                                  // warp uniform
-        int m = 0;
-        if (colok && y >= 2 && y < p.h - 2)
-            m = comb_px<PIX, GAMMA>(prev, next, s_lut, p, (size_t)y * p.pitch + x, c[r], c[r + 1], c[r + 2], c[r + 3], c[r + 4],
-                                    g[r], g[r + 1], g[r + 2], g[r + 3], g[r + 4]);
-        const uint32_t word = __ballot_sync(0xffffffffu, m != 0);
-        if (lane == 0) bits[(size_t)(y + kGuard) * wpitch + 1 + wx] = word;
-    }
-}
+enum { OP_CLASSIC = 0, OP_HV = 1, OP_ERODE = 2, OP_DILATE = 3 };
 
 // the first gate of the decision (comb_detect_template.c:300-312): both vertical neighbours differ from the sample in the
 // same direction by more than the threshold.  Only samples that pass need the previous / next frame at all.
@@ -402,12 +112,13 @@ __device__ __forceinline__ int comb_rest(const CombParams &p, int pu2, int pu1, 
     return 0;
 }
 
-// Round 2 variant of the mask kernel, three phases instead of a row loop that stalls on its own loads: (1) the spatial gate of
-// all kMaskRows rows from the column segment in registers; (2) every previous / next-frame sample some gated row of this lane
-// needs (rows y-1, y, y+1: consecutive output rows share two of three) issued back to back as predicated loads, then their
-// gamma lookups; (3) the motion tests and the metric, ballots and stores.  Round 1 let each gated row fetch its own six
-// samples inside the row loop: up to 16 exposed DRAM round trips per lane (8.3 long-scoreboard stalls per issue,
-// profiles/r02_comb_mask_ncu.json) and every sample fetched up to three times.
+// The mask kernel, in three phases rather than a row loop that stalls on its own loads: (1) the spatial gate of all kMaskRows
+// rows from the column segment in registers; (2) every previous / next-frame sample some gated row of this lane needs (rows
+// y-1, y, y+1: consecutive output rows share two of three) issued back to back as predicated loads, then their gamma
+// lookups; (3) the motion tests and the metric, ballots and stores.  A row loop in which each gated row fetches its own six
+// samples has up to 16 exposed DRAM round trips per lane (8.3 long-scoreboard stalls per issue,
+// profiles/r02_comb_mask_ncu.json) and fetches every sample up to three times: 49.2 us against 37.8 us for the 4K 10-bit
+// luma plane (profiles/r02_comb_mask2_ncu.json).
 template <typename PIX, bool GAMMA>
 __global__ void __launch_bounds__(256) comb_mask_bits2_kernel(const PIX *__restrict__ prev, const PIX *__restrict__ cur,
                                                              const PIX *__restrict__ next, uint32_t *__restrict__ bits,
@@ -635,9 +346,9 @@ struct hbcu_comb_detect_s
     std::vector<uint8_t *> luma;
     std::vector<int64_t> index;
     std::vector<cudaEvent_t> ev_upload, ev_readers;
-    uint8_t *d_mask, *d_scored;
-    uint32_t *d_bits, *d_fbits;      // raw / filtered bit planes (bit-packed path)
-    int wpitch, nwords, use_bits;
+    uint8_t *d_mask, *d_scored;      // byte masks unpacked from the bit planes for hbcu_comb_detect_masks
+    uint32_t *d_bits, *d_fbits;      // raw / filtered bit planes
+    int wpitch, nwords;
     float *d_lut;
     int nres;
     int *d_flags;            // nres ints
@@ -692,8 +403,6 @@ int hbcu_comb_detect_create(hbcu_comb_detect_t **out, const hbcu_comb_detect_con
     h->d_bits = h->d_fbits = nullptr;
     h->nwords = (cfg->width + 31) / 32;
     h->wpitch = h->nwords + 2;
-    h->use_bits = 1;
-    if (const char *e = getenv("HBCU_COMB_IMPL")) h->use_bits = strcmp(e, "bytes") != 0;      // A/B hook: the byte-mask kernels
     h->d_lut = nullptr;
     h->d_flags = nullptr;
     h->h_flags = nullptr;
@@ -842,107 +551,45 @@ int hbcu_comb_detect_run(hbcu_comb_detect_t *h, int64_t prev, int64_t cur, int64
 
     HBCU_CHECK(cudaMemsetAsync(h->d_flags + r, 0, sizeof(int), h->s_compute));
     // block grid: y = k*bh while y + bh <= height; x = j*bw while x < width - bw   (comb_detect.c:238-240)
-    const int bw_ = c.block_width < c.width ? c.block_width : c.width;
-    const int bh_ = c.block_height < c.height ? c.block_height : c.height;
-    const int nby_ = c.height / bh_;
-    const int nbx_ = (c.width - bw_ + bw_ - 1) / bw_;       // number of j with j*bw < width - bw
-    if (h->use_bits)
+    const int bw = c.block_width < c.width ? c.block_width : c.width;
+    const int bh = c.block_height < c.height ? c.block_height : c.height;
+    const int nby = c.height / bh;
+    const int nbx = (c.width - bw + bw - 1) / bw;       // number of j with j*bw < width - bw
+    const bool gamma = (c.mode & 1) != 0;
+    const size_t lut_bytes = gamma ? (size_t)p.lut_size * sizeof(float) : 0;
+    if (lut_bytes > 48 * 1024)
     {
-        const bool gamma = (c.mode & 1) != 0;
-        const size_t lut_bytes = gamma ? (size_t)p.lut_size * sizeof(float) : 0;
-        if (lut_bytes > 48 * 1024)
-        {
-            set_error("comb_detect: gamma table for depth %d does not fit shared memory", c.depth);
-            return -1;
-        }
-        dim3 mgrid((h->nwords + 7) / 8, (c.height + kMaskRows - 1) / kMaskRows);
-        // three-phase kernel by default (37.8 us against 49.2 us for the 4K 10-bit luma plane, profiles/r02_comb_mask2_ncu.json);
-        // HBCU_COMB_MASK=1 selects the round-1 row-loop kernel (A/B, tests)
-        static const int mask_impl = getenv("HBCU_COMB_MASK") ? atoi(getenv("HBCU_COMB_MASK")) : 2;
-#define MASK(K, PIX, A, B, D)                                                                                               \
-        do {                                                                                                                \
-            if (gamma) K<PIX, true><<<mgrid, 256, lut_bytes, h->s_compute>>>(A, B, D, h->d_bits, h->wpitch, p);           \
-            else       K<PIX, false><<<mgrid, 256, 0, h->s_compute>>>(A, B, D, h->d_bits, h->wpitch, p);                  \
-        } while (0)
-        if (h->bps == 1)
-        {
-            if (mask_impl == 2) MASK(comb_mask_bits2_kernel, uint8_t, pl[0], pl[1], pl[2]);
-            else                MASK(comb_mask_bits_kernel, uint8_t, pl[0], pl[1], pl[2]);
-        }
-        else
-        {
-            const uint16_t *a = (const uint16_t *)pl[0], *b = (const uint16_t *)pl[1], *d = (const uint16_t *)pl[2];
-            if (mask_impl == 2) MASK(comb_mask_bits2_kernel, uint16_t, a, b, d);
-            else                MASK(comb_mask_bits_kernel, uint16_t, a, b, d);
-        }
-#undef MASK
-        hbcu::count_launch();
-        HBCU_CHECK(cudaGetLastError());
-        const bool filtered = (c.mode & 2) != 0;
-        const uint32_t *scored = h->d_bits;
-        if (filtered)
-        {
-            dim3 fgrid((h->nwords + BT_W - 1) / BT_W, (c.height + BT_R - 1) / BT_R);
-            comb_filter_bits_kernel<<<fgrid, 256, 0, h->s_compute>>>(h->d_bits, h->d_fbits, h->wpitch, h->nwords, c.width, c.height, c.filter_mode);
-            hbcu::count_launch();
-            HBCU_CHECK(cudaGetLastError());
-            scored = h->d_fbits;
-        }
-        if (nbx_ > 0 && nby_ > 0)
-        {
-            const int warps = nbx_ * nby_;
-            comb_score_bits_kernel<<<(warps * 32 + 127) / 128, 128, 0, h->s_compute>>>(scored, h->wpitch, c.width, c.height, bw_, bh_, nbx_, nby_,
-                                                                                        c.block_threshold, filtered ? 1 : 0, h->d_flags + r);
-            hbcu::count_launch();
-            HBCU_CHECK(cudaGetLastError());
-        }
+        set_error("comb_detect: gamma table for depth %d does not fit shared memory", c.depth);
+        return -1;
     }
-    else
+    dim3 mgrid((h->nwords + 7) / 8, (c.height + kMaskRows - 1) / kMaskRows);
+#define MASK(PIX, A, B, D)                                                                                                  \
+    do {                                                                                                                    \
+        if (gamma) comb_mask_bits2_kernel<PIX, true><<<mgrid, 256, lut_bytes, h->s_compute>>>(A, B, D, h->d_bits, h->wpitch, p); \
+        else       comb_mask_bits2_kernel<PIX, false><<<mgrid, 256, 0, h->s_compute>>>(A, B, D, h->d_bits, h->wpitch, p);        \
+    } while (0)
+    if (h->bps == 1) MASK(uint8_t, pl[0], pl[1], pl[2]);
+    else             MASK(uint16_t, (const uint16_t *)pl[0], (const uint16_t *)pl[1], (const uint16_t *)pl[2]);
+#undef MASK
+    hbcu::count_launch();
+    HBCU_CHECK(cudaGetLastError());
+    const bool filtered = (c.mode & 2) != 0;
+    const uint32_t *scored = h->d_bits;
+    if (filtered)
     {
-        dim3 blk(64, 4), grid((c.width + 63) / 64, (c.height + 3) / 4);
-        const bool gamma = (c.mode & 1) != 0;
-        const size_t lut_bytes = gamma ? (size_t)p.lut_size * sizeof(float) : 0;
-        if (lut_bytes > 48 * 1024)
-        {
-            set_error("comb_detect: gamma table for depth %d does not fit shared memory", c.depth);
-            return -1;
-        }
-        if (h->bps == 1)
-        {
-            if (gamma) comb_mask_kernel<uint8_t, true><<<grid, blk, lut_bytes, h->s_compute>>>(pl[0], pl[1], pl[2], h->d_mask, h->mpitch, p);
-            else       comb_mask_kernel<uint8_t, false><<<grid, blk, 0, h->s_compute>>>(pl[0], pl[1], pl[2], h->d_mask, h->mpitch, p);
-        }
-        else
-        {
-            const uint16_t *a = (const uint16_t *)pl[0], *b = (const uint16_t *)pl[1], *d = (const uint16_t *)pl[2];
-            if (gamma) comb_mask_kernel<uint16_t, true><<<grid, blk, lut_bytes, h->s_compute>>>(a, b, d, h->d_mask, h->mpitch, p);
-            else       comb_mask_kernel<uint16_t, false><<<grid, blk, 0, h->s_compute>>>(a, b, d, h->d_mask, h->mpitch, p);
-        }
+        dim3 fgrid((h->nwords + BT_W - 1) / BT_W, (c.height + BT_R - 1) / BT_R);
+        comb_filter_bits_kernel<<<fgrid, 256, 0, h->s_compute>>>(h->d_bits, h->d_fbits, h->wpitch, h->nwords, c.width, c.height, c.filter_mode);
         hbcu::count_launch();
         HBCU_CHECK(cudaGetLastError());
-        const bool filtered = (c.mode & 2) != 0;
-        const uint8_t *scored = h->d_mask;
-        if (filtered)
-        {
-            dim3 fgrid((c.width + FT_W - 1) / FT_W, (c.height + FT_H - 1) / FT_H);
-            comb_filter_kernel<<<fgrid, 256, 0, h->s_compute>>>(h->d_mask, h->d_scored, h->mpitch, c.width, c.height, c.filter_mode);
-            hbcu::count_launch();
-            HBCU_CHECK(cudaGetLastError());
-            scored = h->d_scored;
-        }
-        // block grid: y = k*bh while y + bh <= height; x = j*bw while x < width - bw   (comb_detect.c:238-240)
-        const int bw = c.block_width < c.width ? c.block_width : c.width;
-        const int bh = c.block_height < c.height ? c.block_height : c.height;
-        const int nby = c.height / bh;
-        const int nbx = (c.width - bw + bw - 1) / bw;       // number of j with j*bw < width - bw
-        if (nbx > 0 && nby > 0)
-        {
-            const int warps = nbx * nby;
-            comb_score_kernel<<<(warps * 32 + 127) / 128, 128, 0, h->s_compute>>>(scored, h->mpitch, c.width, c.height, bw, bh, nbx, nby,
-                                                                                   c.block_threshold, filtered ? 1 : 0, h->d_flags + r);
-            hbcu::count_launch();
-            HBCU_CHECK(cudaGetLastError());
-        }
+        scored = h->d_fbits;
+    }
+    if (nbx > 0 && nby > 0)
+    {
+        const int warps = nbx * nby;
+        comb_score_bits_kernel<<<(warps * 32 + 127) / 128, 128, 0, h->s_compute>>>(scored, h->wpitch, c.width, c.height, bw, bh, nbx, nby,
+                                                                                    c.block_threshold, filtered ? 1 : 0, h->d_flags + r);
+        hbcu::count_launch();
+        HBCU_CHECK(cudaGetLastError());
     }
     HBCU_CHECK(cudaMemcpyAsync(h->h_flags + r, h->d_flags + r, sizeof(int), cudaMemcpyDeviceToHost, h->s_compute));
     HBCU_CHECK(cudaEventRecord(h->ev_result[r], h->s_compute));
@@ -975,19 +622,12 @@ int hbcu_comb_detect_masks(hbcu_comb_detect_t *h, uint8_t *raw, uint8_t *scored)
     HBCU_CHECK(cudaSetDevice(h->cfg.device));
     HBCU_CHECK(cudaStreamSynchronize(h->s_compute));
     const size_t w = h->cfg.width, hh = h->cfg.height;
-    if (h->use_bits)
-    {
-        dim3 blk(64, 4), grid(((int)w + 63) / 64, ((int)hh + 3) / 4);
-        comb_unpack_bits_kernel<<<grid, blk, 0, h->s_compute>>>(h->d_bits, h->wpitch, h->d_mask, h->mpitch, (int)w, (int)hh);
-        comb_unpack_bits_kernel<<<grid, blk, 0, h->s_compute>>>((h->cfg.mode & 2) ? h->d_fbits : h->d_bits, h->wpitch, h->d_scored, h->mpitch, (int)w, (int)hh);
-        HBCU_CHECK(cudaStreamSynchronize(h->s_compute));
-        if (raw) HBCU_CHECK(cudaMemcpy2D(raw, w, h->d_mask, h->mpitch, w, hh, cudaMemcpyDeviceToHost));
-        if (scored) HBCU_CHECK(cudaMemcpy2D(scored, w, h->d_scored, h->mpitch, w, hh, cudaMemcpyDeviceToHost));
-        return 0;
-    }
+    dim3 blk(64, 4), grid(((int)w + 63) / 64, ((int)hh + 3) / 4);
+    comb_unpack_bits_kernel<<<grid, blk, 0, h->s_compute>>>(h->d_bits, h->wpitch, h->d_mask, h->mpitch, (int)w, (int)hh);
+    comb_unpack_bits_kernel<<<grid, blk, 0, h->s_compute>>>((h->cfg.mode & 2) ? h->d_fbits : h->d_bits, h->wpitch, h->d_scored, h->mpitch, (int)w, (int)hh);
+    HBCU_CHECK(cudaStreamSynchronize(h->s_compute));
     if (raw) HBCU_CHECK(cudaMemcpy2D(raw, w, h->d_mask, h->mpitch, w, hh, cudaMemcpyDeviceToHost));
-    if (scored)
-        HBCU_CHECK(cudaMemcpy2D(scored, w, (h->cfg.mode & 2) ? h->d_scored : h->d_mask, h->mpitch, w, hh, cudaMemcpyDeviceToHost));
+    if (scored) HBCU_CHECK(cudaMemcpy2D(scored, w, h->d_scored, h->mpitch, w, hh, cudaMemcpyDeviceToHost));
     return 0;
 }
 

@@ -46,24 +46,13 @@ struct LapFrame
     int max_value;
 };
 
-// int -> double without the conversion instruction: I2F.F64 issues at 15.7 lanes/clk/SM on B200, DADD at 63.8
-// (tools/latency_bench.cu).  0x43300000:lo is 2^52 + lo; subtracting the bias back is exact.
-__device__ __forceinline__ double exact_i2d(int v)
-{
-    return __dadd_rn(__hiloint2double(0x43300000, v ^ (int)0x80000000), -4503601774854144.0);      // -(2^52 + 2^31)
-}
-__device__ __forceinline__ double exact_u2d(int v)                                                     // 0 <= v < 2^31
-{
-    return __dadd_rn(__hiloint2double(0x43300000, v), -4503599627370496.0);                           // -2^52
-}
-
-template <typename PIX, typename ACC, bool MAGIC>
+template <typename PIX, typename ACC>
 __device__ __forceinline__ int lap_finish(int acc, int s0, double coef, double strength, int max_value)
 {
     // the sharpening term exactly as the reference writes it (lapsharp.c:160-176): ACC wrap, double arithmetic,
     // truncation toward zero, ACC wrap again, clamp
     ACC pixel = (ACC)acc;
-    const double dp = MAGIC ? exact_i2d((int)pixel) : (double)pixel, ds = MAGIC ? exact_u2d(s0) : (double)s0;
+    const double dp = (double)pixel, ds = (double)s0;
     const double t = __dmul_rn(__dsub_rn(__dmul_rn(dp, coef), ds), strength);
     pixel = (ACC)((int)(ACC)(int)t + s0);
     int v = pixel;
@@ -73,7 +62,7 @@ __device__ __forceinline__ int lap_finish(int acc, int s0, double coef, double s
 
 // one thread = 4 adjacent pixels of one row.  Interior groups read each of their SIZE input rows as three (8-bit) or four
 // (16-bit) aligned 32-bit words through the read-only path and pick the SIZE+3 samples out of them.
-template <typename PIX, typename ACC, int KID, bool VEC, bool MAGIC>
+template <typename PIX, typename ACC, int KID, bool VEC>
 __device__ __forceinline__ void lap_px4(const LapPlane &p, int max_value, int x0, int y)
 {
     constexpr int SIZE = KID < 2 ? 3 : 5;
@@ -143,7 +132,7 @@ __device__ __forceinline__ void lap_px4(const LapPlane &p, int max_value, int x0
             }
         }
 #pragma unroll
-        for (int i = 0; i < 4; i++) out[i] = lap_finish<PIX, ACC, MAGIC>(acc[i], s0[i], p.coef, p.strength, max_value);
+        for (int i = 0; i < 4; i++) out[i] = lap_finish<PIX, ACC>(acc[i], s0[i], p.coef, p.strength, max_value);
     }
     else
     {
@@ -167,7 +156,7 @@ __device__ __forceinline__ void lap_px4(const LapPlane &p, int max_value, int x0
                     const int c = K.v[(j - offset_min) * SIZE + k - offset_min];
                     if (c != 0) acc += c * (int)src[(size_t)(y + j) * spitch + (x + k)];
                 }
-            out[i] = lap_finish<PIX, ACC, MAGIC>(acc, s0, p.coef, p.strength, max_value);
+            out[i] = lap_finish<PIX, ACC>(acc, s0, p.coef, p.strength, max_value);
         }
     }
     PIX *drow = (PIX *)p.dst + (size_t)y * p.dpitch;
@@ -208,7 +197,7 @@ __host__ __device__ constexpr int lap_tap_word(int j, int k)
 // shift of two loaded words and `dp4a` applies that kernel row's taps in one instruction (9 / 25 multiply-adds per pixel
 // become 3 / 5+).  Accumulating in 32 bits and wrapping to ACC once equals the reference's wrap after every tap
 // (lapsharp.c:150-158: modular arithmetic).  Every other tile goes row by row through lap_px4.
-template <typename PIX, typename ACC, int KID, bool VEC, int R, bool MAGIC>
+template <typename PIX, typename ACC, int KID, bool VEC, int R>
 __device__ __forceinline__ void lap_tile(const LapPlane &p, int max_value, int x0, int y0)
 {
     constexpr int SIZE = KID < 2 ? 3 : 5;
@@ -223,7 +212,7 @@ __device__ __forceinline__ void lap_tile(const LapPlane &p, int max_value, int x
     {
 #pragma unroll 1
         for (int r = 0; r < R; r++)
-            if (y0 + r < height) lap_px4<PIX, ACC, KID, VEC, MAGIC>(p, max_value, x0, y0 + r);
+            if (y0 + r < height) lap_px4<PIX, ACC, KID, VEC>(p, max_value, x0, y0 + r);
         return;
     }
     const PIX *src = (const PIX *)p.src + (size_t)(y0 + offset_min) * spitch + x0;
@@ -273,7 +262,7 @@ __device__ __forceinline__ void lap_tile(const LapPlane &p, int max_value, int x
             int o[4];
 #pragma unroll
             for (int i = 0; i < 4; i++)
-                o[i] = lap_finish<PIX, ACC, MAGIC>(acc[r][i], (int)((centre[r] >> (8 * i)) & 0xffu), p.coef, p.strength, max_value);
+                o[i] = lap_finish<PIX, ACC>(acc[r][i], (int)((centre[r] >> (8 * i)) & 0xffu), p.coef, p.strength, max_value);
             *reinterpret_cast<uchar4 *>(drow + (size_t)r * p.dpitch) = make_uchar4(o[0], o[1], o[2], o[3]);
         }
     }
@@ -318,7 +307,7 @@ __device__ __forceinline__ void lap_tile(const LapPlane &p, int max_value, int x
             for (int i = 0; i < 4; i++)
             {
                 const uint32_t w = centre[r][i >> 1];
-                o[i] = lap_finish<PIX, ACC, MAGIC>(acc[r][i], (int)((i & 1) ? (w >> 16) : (w & 0xffffu)), p.coef, p.strength, max_value);
+                o[i] = lap_finish<PIX, ACC>(acc[r][i], (int)((i & 1) ? (w >> 16) : (w & 0xffffu)), p.coef, p.strength, max_value);
             }
             *reinterpret_cast<ushort4 *>(drow + (size_t)r * p.dpitch) = make_ushort4(o[0], o[1], o[2], o[3]);
         }
@@ -327,7 +316,7 @@ __device__ __forceinline__ void lap_tile(const LapPlane &p, int max_value, int x
 
 // all three planes of a frame in ONE launch (blockIdx.z = plane; the grid is sized for luma, chroma CTAs beyond their plane
 // leave at once): three launches per frame ended in three partial waves
-template <typename PIX, typename ACC, bool VEC, int R, int MINB, bool MAGIC>
+template <typename PIX, typename ACC, bool VEC, int R, int MINB>
 __global__ void __launch_bounds__(256, MINB) lapsharp_kernel(const __grid_constant__ LapFrame f)
 {
     const LapPlane &p = f.pl[blockIdx.z];
@@ -335,10 +324,10 @@ __global__ void __launch_bounds__(256, MINB) lapsharp_kernel(const __grid_consta
     if (x0 >= p.width || y0 >= p.height) return;
     switch (p.kid)                                   // uniform per CTA
     {
-        case 0:  lap_tile<PIX, ACC, 0, VEC, R, MAGIC>(p, f.max_value, x0, y0); break;
-        case 1:  lap_tile<PIX, ACC, 1, VEC, R, MAGIC>(p, f.max_value, x0, y0); break;
-        case 2:  lap_tile<PIX, ACC, 2, VEC, R, MAGIC>(p, f.max_value, x0, y0); break;
-        default: lap_tile<PIX, ACC, 3, VEC, R, MAGIC>(p, f.max_value, x0, y0); break;
+        case 0:  lap_tile<PIX, ACC, 0, VEC, R>(p, f.max_value, x0, y0); break;
+        case 1:  lap_tile<PIX, ACC, 1, VEC, R>(p, f.max_value, x0, y0); break;
+        case 2:  lap_tile<PIX, ACC, 2, VEC, R>(p, f.max_value, x0, y0); break;
+        default: lap_tile<PIX, ACC, 3, VEC, R>(p, f.max_value, x0, y0); break;
     }
 }
 
@@ -396,17 +385,15 @@ int launch_frame(hbcu_lapsharp_s *h, const void *const src[3], const int spitch_
     const Geom &g0 = h->g[0];
     const bool vec = f.pl[0].vec && f.pl[1].vec && f.pl[2].vec;
     // 4 rows per thread at 4 CTAs per SM (64 registers) measured best of {2, 4, 8 rows} x {2..6 CTAs}: 47.7k frames/s against
-    // 42.7k at 2 CTAs per SM (profiles/r02_lapsharp_variants.txt).  HBCU_LAP_VARIANT=8: the exact_i2d arithmetic instead of
-    // the conversion instructions -- measured SLOWER (43.9k against 46.8k on the same box: the two extra DADD and the xor cost
-    // more issue slots than the quarter-rate I2F.F64 costs pipe time), kept for the A/B only.
-    static const int variant = getenv("HBCU_LAP_VARIANT") ? atoi(getenv("HBCU_LAP_VARIANT")) : 0;
+    // 42.7k at 2 CTAs per SM (profiles/r02_lapsharp_variants.txt).  The int -> double conversions stay instructions: building
+    // the double from its bit pattern (2^52 + v, then subtract the bias) measured slower, 43.9k against 46.8k on the same box
+    // (the two extra DADD and the xor cost more issue slots than the quarter-rate I2F.F64 costs pipe time).
     constexpr int R = 4;
     dim3 blk(32, 8), grid(((g0.w + 3) / 4 + 31) / 32, (g0.h + 8 * R - 1) / (8 * R), 3);
 #define LAP(PIX, ACC, MB)                                                                                          \
     do {                                                                                                           \
-        if (!vec)              lapsharp_kernel<PIX, ACC, false, R, 2, false><<<grid, blk, 0, h->s_compute>>>(f);   \
-        else if (variant == 8) lapsharp_kernel<PIX, ACC, true, R, MB, true><<<grid, blk, 0, h->s_compute>>>(f);    \
-        else                   lapsharp_kernel<PIX, ACC, true, R, MB, false><<<grid, blk, 0, h->s_compute>>>(f);   \
+        if (!vec) lapsharp_kernel<PIX, ACC, false, R, 2><<<grid, blk, 0, h->s_compute>>>(f);                         \
+        else      lapsharp_kernel<PIX, ACC, true, R, MB><<<grid, blk, 0, h->s_compute>>>(f);                          \
     } while (0)
     if (h->bps == 1) LAP(uint8_t, int16_t, 4);
     else             LAP(uint16_t, int32_t, 3);          // 85 registers: the 16-bit tile spills at 64

@@ -3,7 +3,8 @@
 // Replaces (reference /root/reference/libhb):
 //   nlmeans_alloc / nlmeans_border      templates/nlmeans_template.c:20-101   -> pad_mirror_kernel
 //   build_integral_scalar / _sse2       templates/nlmeans_template.c:545-591, nlmeans_x86.c:20-149
-//   nlmeans_plane                       templates/nlmeans_template.c:593-717  -> nlmeans_tiled_kernel
+//   nlmeans_plane                       templates/nlmeans_template.c:593-717  -> nlmeans_v3_kernel, nlmeans_v3w_kernel,
+//                                                                               nlmeans_tiled_kernel, nlmeans_generic_kernel
 //   taskset fork/join per frame         nlmeans.c:546-597                      -> stream/event ordering
 //
 // Numeric contract (SURVEY.md appendix B): patch distances are exact integers
@@ -21,8 +22,18 @@
 // thread marches down a 4-pixel-wide column strip keeping, per displacement,
 // the vertical running sum of horizontal patch-row sums in registers (the
 // n-row history lives in registers too), three horizontal displacements per
-// pass; weight/pixel accumulators live in shared memory.  HBM traffic is the
-// algorithmic minimum: every input tile is read once per output tile.
+// pass.  HBM traffic is the algorithmic minimum: every input tile is read once
+// per output tile.  pick_kernel() chooses per plane:
+//   nlmeans_v3_kernel       8-bit planes (nlmeans_v3.cuh): packed-byte patch
+//                           distances, weight/pixel accumulators in tensor
+//                           memory, all planes of a frame in one launch; a
+//                           variant takes the distances from prefiltered planes
+//   nlmeans_v3w_kernel      9/10-bit planes, fp32-exact patch distances
+//   nlmeans_tiled_kernel    integer arithmetic, accumulators in shared memory:
+//                           16-bit samples above 10 bit, ranges the v3 kernels
+//                           are not built for (range 1)
+//   nlmeans_generic_kernel  one thread per pixel: patch/range beyond the tile
+//                           halo, prefilters the v3 variant does not take
 #include "hbcu_common.h"
 #include "hbcu_frames.h"
 #include "../../include/hbcu.h"
@@ -43,7 +54,7 @@ using hbcu::set_error;
 
 constexpr int kBorder    = 16;    // ((n+2)/2+15)/16*16 for every preset (nlmeans.c:529)
 constexpr int kMaxFrames = 32;    // NLMEANS_FRAMES_MAX
-constexpr int kMaxDevices = 64;   // per-device launch configuration flags (power of two)
+constexpr int kMaxDevices = 64;   // peer-access flags per ordered device pair (power of two)
 constexpr int kTileW     = 128;
 constexpr int kHalo      = 8;     // vertical halo of the shared-memory tiles (>= n/2 + r/2)
 // Horizontal halo.  Measured on B200 (tools/tma_test.cu): cp.async.bulk.tensor raises
@@ -61,9 +72,10 @@ constexpr int kTraceFrames = 512;
 
 constexpr int kMaxTiledFrames = 8; // temporal depth the tiled kernel takes (tensor maps travel as kernel parameters)
 
-// largest sample value the fp32-exact 16-bit kernel accepts (10-bit video), and the bits above it in a packed pair
-constexpr unsigned kFast16Max      = 1023u;
-constexpr unsigned kFast16HighBits = 0xFC00FC00u;
+// largest sample value the fp32-exact 16-bit kernel (nlmeans_v3w_kernel) accepts (10-bit video), and the bits above it
+// in a packed pair
+constexpr unsigned kMax10Bit       = 1023u;
+constexpr unsigned kAbove10BitBits = 0xFC00FC00u;
 
 struct KernelParams
 {
@@ -103,7 +115,7 @@ __global__ void pad_mirror_kernel(const PIX *__restrict__ src, int spitch, int w
     y = min(max(y, 0), h - 1);
     const PIX v = src[(size_t)y * spitch + x];
     dst[(size_t)by * bpitch + bx] = v;
-    if (sizeof(PIX) == 2 && range_flag != nullptr && (unsigned)v > kFast16Max) atomicOr(range_flag, 1u);
+    if (sizeof(PIX) == 2 && range_flag != nullptr && (unsigned)v > kMax10Bit) atomicOr(range_flag, 1u);
 }
 
 // 16 bytes per thread: interior chunks are straight uint4 copies, the chunks that touch the mirror border go element by element
@@ -126,8 +138,8 @@ __global__ void __launch_bounds__(256) pad_mirror_vec_kernel(const PIX *__restri
     {
         const uint4 v = *reinterpret_cast<const uint4 *>(srow + (bx0 - border));
         *reinterpret_cast<uint4 *>(drow + bx0) = v;
-        // samples above kFast16Max in a 16-bit plane: tell the fast 10-bit kernel to stand down (see nlmeans_fast16_kernel)
-        if (sizeof(PIX) == 2 && range_flag != nullptr && ((v.x | v.y | v.z | v.w) & kFast16HighBits) != 0u) atomicOr(range_flag, 1u);
+        // samples above kMax10Bit in a 16-bit plane: tell the 10-bit kernel to stand down (see nlmeans_v3w_kernel)
+        if (sizeof(PIX) == 2 && range_flag != nullptr && ((v.x | v.y | v.z | v.w) & kAbove10BitBits) != 0u) atomicOr(range_flag, 1u);
         return;
     }
     bool bad = false;
@@ -141,7 +153,7 @@ __global__ void __launch_bounds__(256) pad_mirror_vec_kernel(const PIX *__restri
         x = min(max(x, 0), w - 1);
         const PIX v = srow[x];
         drow[bx] = v;
-        bad |= sizeof(PIX) == 2 && (unsigned)v > kFast16Max;
+        bad |= sizeof(PIX) == 2 && (unsigned)v > kMax10Bit;
     }
     if (bad && range_flag != nullptr) atomicOr(range_flag, 1u);
 }
@@ -540,10 +552,10 @@ struct TiledParams
 {
     KernelParams k;
     CUtensorMap  maps[kMaxTiledFrames];   // one TMA descriptor per frame of the temporal window
-    const unsigned *only_if_flag;         // when set: run only if *only_if_flag != 0 (stand-in for the fast 16-bit kernel)
+    const unsigned *only_if_flag;         // when set: run only if *only_if_flag != 0 (stand-in for nlmeans_v3w_kernel)
 };
 
-// The fast 8-bit kernel takes up to three planes in ONE launch (tiles of Y, U and V in one grid):
+// The v3 kernels take up to three planes in ONE launch (tiles of Y, U and V in one grid):
 // three separate launches end in three partial waves (510 + 135 + 135 CTAs on 148 SMs = 6 rounds),
 // one launch of all tiles needs 5.
 struct FusedParams
@@ -554,7 +566,7 @@ struct FusedParams
     KernelParams k[3];
     CUtensorMap  maps[3][kMaxTiledFrames];
     CUtensorMap  maps_pre[3][kMaxTiledFrames];   // the pre-denoised planes (prefilter variant of the v3 kernel only)
-    const unsigned *range_flag;           // 16-bit fast kernel: non-zero = some sample exceeded kFast16Max, do nothing
+    const unsigned *range_flag;           // nlmeans_v3w_kernel: non-zero = some sample exceeded kMax10Bit, do nothing
 };
 
 template <typename PIX, int NH, int TH>
@@ -661,15 +673,11 @@ __global__ void __launch_bounds__(kThreads, 1) nlmeans_tiled_kernel(const __grid
 }
 
 // ---------------------------------------------------------------------------
-// Fast 8-bit kernel (v2).  Same tiling and the same arithmetic results as the
-// kernel above, re-expressed for the B200 issue ports measured in
+// v3 kernels (nlmeans_v3.cuh).  Same tiling and the same arithmetic results as
+// the kernel above, re-expressed for the B200 issue ports measured in
 // profiles/r01_microbench_instruction_throughput.txt:
 //   * FADD/FMUL/FFMA issue at 4 warp-instr/clk/SM, integer ALU ops (PRMT, LOP3,
 //     IADD3, IMAD) at 2, F2I / I2F.U8 at 0.5, LDS at ~1.
-//   * For 8-bit pixels every quantity of the patch distance is an integer
-//     below 2^24 (7*7*255^2 = 3.2M), so it is computed in fp32 EXACTLY: the
-//     squared difference is one FFMA into a running prefix sum, the patch-row
-//     sum one FADD, the vertical window two FADDs.  No int->float conversion.
 //   * Pixels are fetched as 32-bit words (conflict-free LDS.32) and unpacked
 //     with PRMT straight into the float 2^23+v (bits 0x4B0000vv): differences
 //     of two such floats are exact.
@@ -677,26 +685,9 @@ __global__ void __launch_bounds__(kThreads, 1) nlmeans_tiled_kernel(const __grid
 //     FMUL.SAT by wfact/128 (power-of-two scaling is exact), FADD.RZ with 2^16
 //     (the mantissa then holds floor(128*t)), and a 129-entry table whose
 //     entries 127 and 128 are 0.  Valid while wfact < 0.99 (then diff >=
-//     diff_max implies idx >= 127); launch_plane() checks it.  No F2I.
+//     diff_max implies idx >= 127); pick_kernel() checks it.  No F2I.
 // ---------------------------------------------------------------------------
 constexpr int kLutEntries = HBCU_NLMEANS_EXPSIZE + 1;
-
-template <int TH>
-struct FastLayout
-{
-    static constexpr int kRows      = TH + 2 * kHalo;
-    static constexpr int kTileBytes = kRows * kTilePW;
-    static constexpr int kAccBytes  = TH * kTileW * (int)sizeof(float);
-    static constexpr int kLutBytes  = kLutEntries * 32 * (int)sizeof(float);
-    static constexpr int kOffCur    = 0;
-    static constexpr int kOffCmp    = kOffCur + kTileBytes;
-    static constexpr int kOffWs     = kOffCmp + kTileBytes;
-    static constexpr int kOffPs     = kOffWs + kAccBytes;
-    static constexpr int kOffLut    = kOffPs + kAccBytes;
-    static constexpr int kOffBar    = kOffLut + kLutBytes;
-    static constexpr int kTotal     = kOffBar + 64;
-    static_assert(kTileBytes % 128 == 0, "TMA destination must stay 128-byte aligned");
-};
 
 // byte k (0..3) of word w as the float 2^23 + value
 __device__ __forceinline__ float byte_as_biased_float(uint32_t w, int k)
@@ -711,747 +702,6 @@ __device__ __forceinline__ float half_as_biased_float(uint32_t w, int k)
 }
 
 #include "nlmeans_v3.cuh"
-
-template <int NH, int TH, int NW, bool ORIGIN>
-__device__ __forceinline__ void nlm_group_fast(const uint32_t *__restrict__ cur, const uint32_t *__restrict__ cmp,
-                                               float *__restrict__ acc_ws, float *__restrict__ acc_ps,
-                                               uint32_t lut_lane_addr, float wscale, double origin_tune,
-                                               int seg_y0, int lane, int dy, int dx0, int ng, int origin_g)
-{
-    constexpr int N   = 2 * NH + 1;
-    constexpr int RS  = TH / NW;
-    constexpr int NA  = 4 + 2 * NH;                 // source values per row
-    constexpr int NB  = NA + kGroup - 1;            // compare values per row
-    constexpr int PW  = kTilePW / 4;                // tile pitch in words
-    constexpr int OA  = (kHaloX - NH) & 3;          // byte offset of a[0] in its first word
-    constexpr int WA0 = (kHaloX - NH) >> 2;         // first word of the a window (relative to lane word)
-    constexpr int NWA = (OA + NA + 3) / 4;
-    constexpr int NWB = (NB + 3) / 4;               // aligned compare words
-    constexpr float kBias = 8388608.0f;             // 2^23
-
-    const int fb  = kHaloX - NH + dx0;              // first compare column relative to the lane's x
-    const int wb0 = fb >> 2;
-    const int ob  = (fb & 3) * 8;                   // funnel shift (bits) that aligns the compare window
-
-    float V[kGroup][4];
-    float hist[N][kGroup][4];
-#pragma unroll
-    for (int g = 0; g < kGroup; g++)
-#pragma unroll
-        for (int i = 0; i < 4; i++)
-        {
-            V[g][i] = 0.f;
-#pragma unroll
-            for (int k = 0; k < N; k++) hist[k][g][i] = 0.f;
-        }
-    // aligned compare words of the last NH rows: they hold the pixels cmp[y+dy][x+dx] of the
-    // output row that completes NH steps after its own compare row was loaded
-    uint32_t delay[NH][NWB];
-#pragma unroll
-    for (int r = 0; r < NH; r++)
-#pragma unroll
-        for (int j = 0; j < NWB; j++) delay[r][j] = 0;
-
-#pragma unroll 1
-    for (int base = -NH; base < RS + NH; base += N)
-    {
-#pragma unroll
-        for (int k = 0; k < N; k++)
-        {
-            const int yy = base + k;
-            if (yy < RS + NH)
-            {
-                const int ty = seg_y0 + yy + kHalo;
-                const uint32_t *aw = cur + ty * PW + lane + WA0;
-                const uint32_t *bw = cmp + (ty + dy) * PW + lane + wb0;
-                uint32_t wa[NWA], wraw[NWB + 1], wbv[NWB];
-#pragma unroll
-                for (int j = 0; j < NWA; j++) wa[j] = aw[j];
-#pragma unroll
-                for (int j = 0; j < NWB + 1; j++) wraw[j] = bw[j];
-#pragma unroll
-                for (int j = 0; j < NWB; j++) wbv[j] = __funnelshift_r(wraw[j], wraw[j + 1], ob);
-
-                float a[NA], b[NB];
-#pragma unroll
-                for (int j = 0; j < NA; j++) a[j] = byte_as_biased_float(wa[(OA + j) >> 2], (OA + j) & 3);
-#pragma unroll
-                for (int j = 0; j < NB; j++) b[j] = byte_as_biased_float(wbv[j >> 2], j & 3);
-
-#pragma unroll
-                for (int g = 0; g < kGroup; g++)
-                {
-                    if (g < ng && (!ORIGIN || g != origin_g))
-                    {
-                        float c[NA + 1];
-                        c[0] = 0.f;
-#pragma unroll
-                        for (int j = 0; j < NA; j++)
-                        {
-                            const float d = __fsub_rn(a[j], b[j + g]);        // exact
-                            c[j + 1] = __fmaf_rn(d, d, c[j]);                  // exact: integers < 2^24
-                        }
-#pragma unroll
-                        for (int i = 0; i < 4; i++)
-                        {
-                            const float hsum = __fsub_rn(c[i + N], c[i]);
-                            V[g][i] = __fadd_rn(V[g][i], __fsub_rn(hsum, hist[k][g][i]));
-                            hist[k][g][i] = hsum;
-                        }
-                    }
-                }
-                if (yy >= NH)
-                {
-                    const int oy = seg_y0 + yy - NH;
-                    float4 ws4 = *reinterpret_cast<float4 *>(acc_ws + oy * kTileW + lane * 4);
-                    float4 ps4 = *reinterpret_cast<float4 *>(acc_ps + oy * kTileW + lane * 4);
-                    float ws[4] = { ws4.x, ws4.y, ws4.z, ws4.w };
-                    float ps[4] = { ps4.x, ps4.y, ps4.z, ps4.w };
-                    // pixel values cmp[oy+dy][x+dx0+g+i] = element NH+g+i of the compare window loaded NH rows ago
-                    float pixv[kGroup + 3];
-#pragma unroll
-                    for (int j = 0; j < kGroup + 3; j++)
-                        pixv[j] = __fsub_rn(byte_as_biased_float(delay[0][(NH + j) >> 2], (NH + j) & 3), kBias);
-#pragma unroll
-                    for (int g = 0; g < kGroup; g++)
-                    {
-                        if (g < ng)
-                        {
-                            if (ORIGIN && g == origin_g)
-                            {
-                                const uint32_t cw = cur[(oy + kHalo) * PW + lane + kHaloX / 4];
-#pragma unroll
-                                for (int i = 0; i < 4; i++)
-                                    add_origin(ws[i], ps[i], origin_tune, (int)((cw >> (8 * i)) & 0xffu));
-                            }
-                            else
-                            {
-#pragma unroll
-                                for (int i = 0; i < 4; i++)
-                                {
-                                    float t, u, wgt;
-                                    asm("mul.rn.sat.f32 %0, %1, %2;" : "=f"(t) : "f"(V[g][i]), "f"(wscale));
-                                    asm("add.rz.f32 %0, %1, 0f47800000;" : "=f"(u) : "f"(t));   // 65536 + floor(128 t)
-                                    const uint32_t addr = (__float_as_uint(u) << 7) + lut_lane_addr;
-                                    asm("ld.shared.f32 %0, [%1];" : "=f"(wgt) : "r"(addr));
-                                    ws[i] = __fadd_rn(ws[i], wgt);
-                                    ps[i] = __fadd_rn(ps[i], __fmul_rn(wgt, pixv[g + i]));
-                                }
-                            }
-                        }
-                    }
-                    *reinterpret_cast<float4 *>(acc_ws + oy * kTileW + lane * 4) = make_float4(ws[0], ws[1], ws[2], ws[3]);
-                    *reinterpret_cast<float4 *>(acc_ps + oy * kTileW + lane * 4) = make_float4(ps[0], ps[1], ps[2], ps[3]);
-                }
-                // advance the delay line
-#pragma unroll
-                for (int r = 0; r + 1 < NH; r++)
-#pragma unroll
-                    for (int j = 0; j < NWB; j++) delay[r][j] = delay[r + 1][j];
-#pragma unroll
-                for (int j = 0; j < NWB; j++) delay[NH - 1][j] = wbv[j];
-            }
-        }
-    }
-}
-
-template <int NH, int TH, int NW, bool ORIGIN>
-__device__ __forceinline__ void nlm_group_dp4a(const uint32_t *__restrict__ cur, const uint32_t *__restrict__ cmp,
-                                               float *__restrict__ acc_ws, float *__restrict__ acc_ps,
-                                               uint32_t lut_lane_addr, float wscale, double origin_tune,
-                                               int seg_y0, int lane, int dy, int dx0, int ng, int origin_g)
-{
-    constexpr int N   = 2 * NH + 1;
-    constexpr int RS  = TH / NW;
-    constexpr int NA  = 4 + 2 * NH;                 // source values per row
-    constexpr int NB  = NA + kGroup - 1;            // compare values per row
-    constexpr int PW  = kTilePW / 4;                // tile pitch in words
-    constexpr int OA  = (kHaloX - NH) & 3;          // byte offset of a[0] in its first word
-    constexpr int WA0 = (kHaloX - NH) >> 2;         // first word of the a window (relative to lane word)
-    constexpr int NWA = (OA + NA + 3) / 4;
-    constexpr int NWB = (NB + 3) / 4;               // aligned compare words
-    constexpr float kBias = 8388608.0f;             // 2^23
-
-    const int fb  = kHaloX - NH + dx0;              // first compare column relative to the lane's x
-    const int wb0 = fb >> 2;
-    const int ob  = (fb & 3) * 8;                   // funnel shift (bits) that aligns the compare window
-
-    int V[kGroup][4];
-    int hist[N][kGroup][4];
-#pragma unroll
-    for (int g = 0; g < kGroup; g++)
-#pragma unroll
-        for (int i = 0; i < 4; i++)
-        {
-            V[g][i] = 0;
-#pragma unroll
-            for (int k = 0; k < N; k++) hist[k][g][i] = 0;
-        }
-    // aligned compare words of the last NH rows: they hold the pixels cmp[y+dy][x+dx] of the
-    // output row that completes NH steps after its own compare row was loaded
-    uint32_t delay[NH][NWB];
-#pragma unroll
-    for (int r = 0; r < NH; r++)
-#pragma unroll
-        for (int j = 0; j < NWB; j++) delay[r][j] = 0;
-
-#pragma unroll 1
-    for (int base = -NH; base < RS + NH; base += N)
-    {
-#pragma unroll
-        for (int k = 0; k < N; k++)
-        {
-            const int yy = base + k;
-            if (yy < RS + NH)
-            {
-                const int ty = seg_y0 + yy + kHalo;
-                const uint32_t *aw = cur + ty * PW + lane + WA0;
-                const uint32_t *bw = cmp + (ty + dy) * PW + lane + wb0;
-                uint32_t wa[NWA], wraw[NWB + 1], wbv[NWB];
-#pragma unroll
-                for (int j = 0; j < NWA; j++) wa[j] = aw[j];
-#pragma unroll
-                for (int j = 0; j < NWB + 1; j++) wraw[j] = bw[j];
-#pragma unroll
-                for (int j = 0; j < NWB; j++) wbv[j] = __funnelshift_r(wraw[j], wraw[j + 1], ob);
-
-                // Patch-row sums straight from the packed bytes: |a-b| for four pixels per VABSDIFF4, sums of
-                // squares over the 2NH+1 byte window per IDP4A (whole words) plus masked IDP4As for the partial
-                // words at both ends.  Integer-exact, no unpacking.
-                constexpr int NWD = (NA + 3) / 4;                    // words holding a[0..NA-1]
-                uint32_t aw4[NWD];
-#pragma unroll
-                for (int w = 0; w < NWD; w++)
-                    aw4[w] = OA ? __funnelshift_r(wa[w], (w + 1 < NWA) ? wa[w + 1] : 0u, 8 * OA) : wa[w];
-#pragma unroll
-                for (int g = 0; g < kGroup; g++)
-                {
-                    if (g < ng && (!ORIGIN || g != origin_g))
-                    {
-                        uint32_t D[NWD];
-#pragma unroll
-                        for (int w = 0; w < NWD; w++)
-                        {
-                            const uint32_t bg = g ? __funnelshift_r(wbv[w], (w + 1 < NWB) ? wbv[w + 1] : 0u, 8 * g) : wbv[w];
-                            D[w] = __vabsdiffu4(aw4[w], bg);
-                        }
-                        uint32_t T[NWD];
-#pragma unroll
-                        for (int w = 0; w < NWD; w++) T[w] = __dp4a(D[w], D[w], 0u);
-#pragma unroll
-                        for (int i = 0; i < 4; i++)
-                        {
-                            // window = bytes i .. i+N-1 of the D stream
-                            uint32_t acc = 0;
-                            bool started = false;
-#pragma unroll
-                            for (int w = 0; w < NWD; w++)
-                            {
-                                const int lo = max(i, 4 * w), hi = min(i + N - 1, 4 * w + 3);
-                                if (lo == 4 * w && hi == 4 * w + 3 && !started) { acc = T[w]; started = true; }
-                            }
-                            bool used_full = false;
-#pragma unroll
-                            for (int w = 0; w < NWD; w++)
-                            {
-                                const int lo = max(i, 4 * w), hi = min(i + N - 1, 4 * w + 3);
-                                if (lo > hi) continue;
-                                if (lo == 4 * w && hi == 4 * w + 3)
-                                {
-                                    if (started && !used_full) { used_full = true; continue; }   // already in acc
-                                    acc = __dp4a(D[w], D[w], acc);
-                                }
-                                else
-                                {
-                                    uint32_t m = 0;
-#pragma unroll
-                                    for (int bb = 0; bb < 4; bb++)
-                                        if (4 * w + bb >= lo && 4 * w + bb <= hi) m |= 0xFFu << (8 * bb);
-                                    acc = __dp4a(D[w] & m, D[w], acc);
-                                }
-                            }
-                            const int hsum = (int)acc;
-                            V[g][i] = V[g][i] + hsum - hist[k][g][i];
-                            hist[k][g][i] = hsum;
-                        }
-                    }
-                }
-                if (yy >= NH)
-                {
-                    const int oy = seg_y0 + yy - NH;
-                    float4 ws4 = *reinterpret_cast<float4 *>(acc_ws + oy * kTileW + lane * 4);
-                    float4 ps4 = *reinterpret_cast<float4 *>(acc_ps + oy * kTileW + lane * 4);
-                    float ws[4] = { ws4.x, ws4.y, ws4.z, ws4.w };
-                    float ps[4] = { ps4.x, ps4.y, ps4.z, ps4.w };
-                    // pixel values cmp[oy+dy][x+dx0+g+i] = element NH+g+i of the compare window loaded NH rows ago
-                    float pixv[kGroup + 3];
-#pragma unroll
-                    for (int j = 0; j < kGroup + 3; j++)
-                        pixv[j] = __fsub_rn(byte_as_biased_float(delay[0][(NH + j) >> 2], (NH + j) & 3), kBias);
-#pragma unroll
-                    for (int g = 0; g < kGroup; g++)
-                    {
-                        if (g < ng)
-                        {
-                            if (ORIGIN && g == origin_g)
-                            {
-                                const uint32_t cw = cur[(oy + kHalo) * PW + lane + kHaloX / 4];
-#pragma unroll
-                                for (int i = 0; i < 4; i++)
-                                    add_origin(ws[i], ps[i], origin_tune, (int)((cw >> (8 * i)) & 0xffu));
-                            }
-                            else
-                            {
-#pragma unroll
-                                for (int i = 0; i < 4; i++)
-                                {
-                                    float t, u, wgt;
-                                    asm("mul.rn.sat.f32 %0, %1, %2;" : "=f"(t) : "f"(__int2float_rn(V[g][i])), "f"(wscale));
-                                    asm("add.rz.f32 %0, %1, 0f47800000;" : "=f"(u) : "f"(t));   // 65536 + floor(128 t)
-                                    const uint32_t addr = (__float_as_uint(u) << 7) + lut_lane_addr;
-                                    asm("ld.shared.f32 %0, [%1];" : "=f"(wgt) : "r"(addr));
-                                    ws[i] = __fadd_rn(ws[i], wgt);
-                                    ps[i] = __fadd_rn(ps[i], __fmul_rn(wgt, pixv[g + i]));
-                                }
-                            }
-                        }
-                    }
-                    *reinterpret_cast<float4 *>(acc_ws + oy * kTileW + lane * 4) = make_float4(ws[0], ws[1], ws[2], ws[3]);
-                    *reinterpret_cast<float4 *>(acc_ps + oy * kTileW + lane * 4) = make_float4(ps[0], ps[1], ps[2], ps[3]);
-                }
-                // advance the delay line
-#pragma unroll
-                for (int r = 0; r + 1 < NH; r++)
-#pragma unroll
-                    for (int j = 0; j < NWB; j++) delay[r][j] = delay[r + 1][j];
-#pragma unroll
-                for (int j = 0; j < NWB; j++) delay[NH - 1][j] = wbv[j];
-            }
-        }
-    }
-}
-
-template <int NH, int TH, int NW, bool DP4A>
-__global__ void __launch_bounds__(NW * 32, 1) nlmeans_fast8_kernel(const __grid_constant__ FusedParams fp)
-{
-    constexpr int kThreads = NW * 32;
-    int pl = 0;
-    while (pl + 1 < fp.nplanes && (int)blockIdx.x >= fp.first_tile[pl + 1]) pl++;
-    const KernelParams &p = fp.k[pl];
-    const CUtensorMap *maps = fp.maps[pl];
-    const int tile = (int)blockIdx.x - fp.first_tile[pl];
-    using L = FastLayout<TH>;
-    extern __shared__ __align__(128) uint8_t smem[];
-    uint8_t *cur  = smem + L::kOffCur;
-    uint8_t *cmp  = smem + L::kOffCmp;
-    float *acc_ws = reinterpret_cast<float *>(smem + L::kOffWs);
-    float *acc_ps = reinterpret_cast<float *>(smem + L::kOffPs);
-    float *lut    = reinterpret_cast<float *>(smem + L::kOffLut);
-    uint64_t *bar = reinterpret_cast<uint64_t *>(smem + L::kOffBar);
-
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int X0 = (tile % fp.tiles_x[pl]) * kTileW, Y0 = (tile / fp.tiles_x[pl]) * TH;
-    const int gx = X0 + kBorder - kHaloX, gy = Y0 + kBorder - kHalo;
-
-    if (tid == 0)
-    {
-        mbar_init(bar, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    uint32_t phase = 0;
-    if (tid == 0)
-    {
-        mbar_expect_tx(bar, L::kTileBytes);
-        tma_load_2d(cur, &maps[0], gx, gy, bar);
-    }
-    for (int i = tid; i < kLutEntries * 32; i += kThreads)
-    {
-        const int e = i >> 5;
-        lut[i] = e < HBCU_NLMEANS_EXPSIZE ? p.exptable[e] : 0.f;
-    }
-    for (int i = tid; i < TH * kTileW; i += kThreads)
-    {
-        acc_ws[i] = 0.f;
-        acc_ps[i] = 0.f;
-    }
-    mbar_wait(bar, phase);
-    phase ^= 1;
-    __syncthreads();
-
-    const int seg_y0 = warp * (TH / NW);
-    const float wscale = p.wfact * 0.0078125f;                         // wfact / 128, exact
-    // shared address of this lane's copy of table entry 0, pre-biased by -(0x47800000 << 7)
-    const uint32_t lut_lane_addr = smem_u32(lut) + (uint32_t)lane * 4u - (0x47800000u << 7);
-    for (int f = 0; f < p.nf; f++)
-    {
-        const uint8_t *B = cur;
-        if (f > 0)
-        {
-            __syncthreads();
-            if (tid == 0)
-            {
-                fence_proxy_async();
-                mbar_expect_tx(bar, L::kTileBytes);
-                tma_load_2d(cmp, &maps[f], gx, gy, bar);
-            }
-            mbar_wait(bar, phase);
-            phase ^= 1;
-            B = cmp;
-        }
-        for (int dy = -p.r_half; dy <= p.r_half; dy++)
-        {
-            for (int dx0 = -p.r_half; dx0 <= p.r_half; dx0 += kGroup)
-            {
-                const int ng = min(kGroup, p.r_half - dx0 + 1);
-                const int origin_g = (f == 0 && dy == 0 && dx0 <= 0 && dx0 + ng > 0) ? -dx0 : -1;
-                // the origin variant (double-precision add of origin_tune) runs for one group per plane;
-                // keeping it out of the common instantiation keeps that loop body small
-                const uint32_t *cw = reinterpret_cast<const uint32_t *>(cur), *bw32 = reinterpret_cast<const uint32_t *>(B);
-                if (DP4A)
-                {
-                    if (origin_g >= 0)
-                        nlm_group_dp4a<NH, TH, NW, true>(cw, bw32, acc_ws, acc_ps, lut_lane_addr, wscale, p.origin_tune, seg_y0, lane, dy, dx0, ng, origin_g);
-                    else
-                        nlm_group_dp4a<NH, TH, NW, false>(cw, bw32, acc_ws, acc_ps, lut_lane_addr, wscale, p.origin_tune, seg_y0, lane, dy, dx0, ng, -1);
-                }
-                else
-                {
-                    if (origin_g >= 0)
-                        nlm_group_fast<NH, TH, NW, true>(cw, bw32, acc_ws, acc_ps, lut_lane_addr, wscale, p.origin_tune, seg_y0, lane, dy, dx0, ng, origin_g);
-                    else
-                        nlm_group_fast<NH, TH, NW, false>(cw, bw32, acc_ws, acc_ps, lut_lane_addr, wscale, p.origin_tune, seg_y0, lane, dy, dx0, ng, -1);
-                }
-            }
-        }
-    }
-
-    const int x = lane * 4;
-    uint8_t *dst = reinterpret_cast<uint8_t *>(p.dst);
-    for (int r = 0; r < TH / NW; r++)
-    {
-        const int oy = seg_y0 + r;
-        const int y = Y0 + oy;
-        if (y >= p.h) break;
-        const float4 ws4 = *reinterpret_cast<const float4 *>(acc_ws + oy * kTileW + x);
-        const float4 ps4 = *reinterpret_cast<const float4 *>(acc_ps + oy * kTileW + x);
-        const float ws[4] = { ws4.x, ws4.y, ws4.z, ws4.w };
-        const float ps[4] = { ps4.x, ps4.y, ps4.z, ps4.w };
-        uint8_t o[4];
-#pragma unroll
-        for (int i = 0; i < 4; i++)
-            o[i] = finish_pixel<uint8_t>(ws[i], ps[i], cur[(oy + kHalo) * kTilePW + x + kHaloX + i]);
-        uint8_t *drow = dst + (size_t)y * p.dpitch + X0 + x;
-        if (X0 + x + 3 < p.w)
-            *reinterpret_cast<uchar4 *>(drow) = make_uchar4(o[0], o[1], o[2], o[3]);
-        else
-        {
-#pragma unroll
-            for (int i = 0; i < 4; i++)
-                if (X0 + x + i < p.w) drow[i] = o[i];
-        }
-    }
-}
-
-// ---------------------------------------------------------------------------
-// Fast kernel for 9/10-bit planes (16-bit containers), patch <= 7.  Same tiling, same results.
-// With samples <= 1023 a squared difference is < 2^20, the prefix sum over the <= 10 values a lane touches
-// per row < 2^24 and one patch-row sum (7 * 1023^2) < 2^23, so the row sums are exact in fp32 (FSUB + FFMA per
-// pixel pair like the 8-bit fp32 variant).  The n x n sum (up to 5.1e7) is not, so the vertical running sum is an
-// integer: hsum + 2^23 carries hsum in its mantissa bits and V += bits(new) - bits(old) is one IADD3 with no
-// unbiasing.  Samples travel as LDS.64 (4 samples; a warp reads 256 contiguous bytes, conflict free) and are
-// unpacked by PRMT into the float 2^23 + v.
-// A 16-bit container can hold samples above 1023.  The border kernel raises a sticky flag when it sees one; this
-// kernel then returns at once and the integer kernel launched right behind it (which returns at once when the
-// flag is clear) does the frame: same output either way, no host round trip.
-// ---------------------------------------------------------------------------
-template <int TH>
-struct Fast16Layout
-{
-    static constexpr int kRows      = TH + 2 * kHalo;
-    static constexpr int kTileBytes = kRows * kTilePW * 2;
-    static constexpr int kAccBytes  = TH * kTileW * (int)sizeof(float);
-    static constexpr int kLutBytes  = kLutEntries * 32 * (int)sizeof(float);
-    static constexpr int kOffCur    = 0;
-    static constexpr int kOffCmp    = kOffCur + kTileBytes;
-    static constexpr int kOffWs     = kOffCmp + kTileBytes;
-    static constexpr int kOffPs     = kOffWs + kAccBytes;
-    static constexpr int kOffLut    = kOffPs + kAccBytes;
-    static constexpr int kOffBar    = kOffLut + kLutBytes;
-    static constexpr int kTotal     = kOffBar + 64;
-    static_assert(kTileBytes % 128 == 0, "TMA destination must stay 128-byte aligned");
-};
-
-template <int NH, int TH, int NW, bool ORIGIN>
-__device__ __forceinline__ void nlm_group_fast16(const uint2 *__restrict__ cur, const uint2 *__restrict__ cmp,
-                                                 float *__restrict__ acc_ws, float *__restrict__ acc_ps,
-                                                 uint32_t lut_lane_addr, float wscale, double origin_tune,
-                                                 int seg_y0, int lane, int dy, int dx0, int ng, int origin_g)
-{
-    constexpr int N   = 2 * NH + 1;
-    constexpr int RS  = TH / NW;
-    constexpr int NA  = 4 + 2 * NH;                 // source samples per row
-    constexpr int NB  = NA + kGroup - 1;            // compare samples per row
-    constexpr int PQ  = kTilePW / 4;                // tile pitch in 4-sample quads (uint2)
-    constexpr int OA  = (kHaloX - NH) & 3;          // sample offset of a[0] in its first quad
-    constexpr int QA0 = (kHaloX - NH) >> 2;         // first quad of the a window (relative to the lane's quad)
-    constexpr int NQA = (OA + NA + 3) / 4;
-    constexpr int NQB = (3 + NB + 3) / 4;           // quads loaded for the compare window (covers any alignment)
-    constexpr int NWB = (NB + 1) / 2;               // aligned compare words (two samples each)
-    constexpr float kBias = 8388608.0f;             // 2^23
-    constexpr int kBiasBits = 0x4B000000;
-    static_assert(NH <= 3, "patch-row sums must stay below 2^23");
-    static_assert(NWB + 2 <= 2 * NQB, "compare window must fit the loaded quads");
-
-    const int fb   = kHaloX - NH + dx0;             // first compare column relative to the lane's x
-    const int qb0  = fb >> 2;
-    const bool odd_word = (fb & 2) != 0;            // the aligned stream starts in the second word of the first quad
-    const int sh   = (fb & 1) * 16;                 // and, for odd fb, half a word further
-
-    int V[kGroup][4];
-    int hist[N][kGroup][4];
-#pragma unroll
-    for (int g = 0; g < kGroup; g++)
-#pragma unroll
-        for (int i = 0; i < 4; i++)
-        {
-            V[g][i] = 0;
-#pragma unroll
-            for (int k = 0; k < N; k++) hist[k][g][i] = kBiasBits;
-        }
-    uint32_t delay[NH][NWB];
-#pragma unroll
-    for (int r = 0; r < NH; r++)
-#pragma unroll
-        for (int j = 0; j < NWB; j++) delay[r][j] = 0;
-
-#pragma unroll 1
-    for (int base = -NH; base < RS + NH; base += N)
-    {
-#pragma unroll
-        for (int k = 0; k < N; k++)
-        {
-            const int yy = base + k;
-            if (yy < RS + NH)
-            {
-                const int ty = seg_y0 + yy + kHalo;
-                const uint2 *aq = cur + ty * PQ + lane + QA0;
-                const uint2 *bq = cmp + (ty + dy) * PQ + lane + qb0;
-                uint32_t wa[2 * NQA], wraw[2 * NQB], wbv[NWB];
-#pragma unroll
-                for (int j = 0; j < NQA; j++)
-                {
-                    const uint2 q = aq[j];
-                    wa[2 * j] = q.x;
-                    wa[2 * j + 1] = q.y;
-                }
-#pragma unroll
-                for (int j = 0; j < NQB; j++)
-                {
-                    const uint2 q = bq[j];
-                    wraw[2 * j] = q.x;
-                    wraw[2 * j + 1] = q.y;
-                }
-                uint32_t wsel[NWB + 1];
-#pragma unroll
-                for (int j = 0; j < NWB + 1; j++) wsel[j] = odd_word ? wraw[j + 1] : wraw[j];
-#pragma unroll
-                for (int j = 0; j < NWB; j++) wbv[j] = __funnelshift_r(wsel[j], wsel[j + 1], sh);
-
-                float a[NA], b[NB];
-#pragma unroll
-                for (int j = 0; j < NA; j++) a[j] = half_as_biased_float(wa[(OA + j) >> 1], (OA + j) & 1);
-#pragma unroll
-                for (int j = 0; j < NB; j++) b[j] = half_as_biased_float(wbv[j >> 1], j & 1);
-
-#pragma unroll
-                for (int g = 0; g < kGroup; g++)
-                {
-                    if (g < ng && (!ORIGIN || g != origin_g))
-                    {
-                        float c[NA + 1];
-                        c[0] = 0.f;
-#pragma unroll
-                        for (int j = 0; j < NA; j++)
-                        {
-                            const float d = __fsub_rn(a[j], b[j + g]);        // exact
-                            c[j + 1] = __fmaf_rn(d, d, c[j]);                  // exact: integers < 2^24
-                        }
-#pragma unroll
-                        for (int i = 0; i < 4; i++)
-                        {
-                            const float hsum = __fsub_rn(c[i + N], c[i]);      // < 2^23
-                            const int hb = __float_as_int(__fadd_rn(hsum, kBias));
-                            V[g][i] = V[g][i] + hb - hist[k][g][i];
-                            hist[k][g][i] = hb;
-                        }
-                    }
-                }
-                if (yy >= NH)
-                {
-                    const int oy = seg_y0 + yy - NH;
-                    float4 ws4 = *reinterpret_cast<float4 *>(acc_ws + oy * kTileW + lane * 4);
-                    float4 ps4 = *reinterpret_cast<float4 *>(acc_ps + oy * kTileW + lane * 4);
-                    float ws[4] = { ws4.x, ws4.y, ws4.z, ws4.w };
-                    float ps[4] = { ps4.x, ps4.y, ps4.z, ps4.w };
-                    // cmp[oy+dy][x+dx0+g+i] = sample NH+g+i of the compare window loaded NH rows ago
-                    float pixv[kGroup + 3];
-#pragma unroll
-                    for (int j = 0; j < kGroup + 3; j++)
-                        pixv[j] = __fsub_rn(half_as_biased_float(delay[0][(NH + j) >> 1], (NH + j) & 1), kBias);
-#pragma unroll
-                    for (int g = 0; g < kGroup; g++)
-                    {
-                        if (g < ng)
-                        {
-                            if (ORIGIN && g == origin_g)
-                            {
-                                const uint2 cq = cur[(oy + kHalo) * PQ + lane + kHaloX / 4];
-                                add_origin(ws[0], ps[0], origin_tune, (int)(cq.x & 0xffffu));
-                                add_origin(ws[1], ps[1], origin_tune, (int)(cq.x >> 16));
-                                add_origin(ws[2], ps[2], origin_tune, (int)(cq.y & 0xffffu));
-                                add_origin(ws[3], ps[3], origin_tune, (int)(cq.y >> 16));
-                            }
-                            else
-                            {
-#pragma unroll
-                                for (int i = 0; i < 4; i++)
-                                {
-                                    float t, u, wgt;
-                                    asm("mul.rn.sat.f32 %0, %1, %2;" : "=f"(t) : "f"(__int2float_rn(V[g][i])), "f"(wscale));
-                                    asm("add.rz.f32 %0, %1, 0f47800000;" : "=f"(u) : "f"(t));   // 65536 + floor(128 t)
-                                    const uint32_t addr = (__float_as_uint(u) << 7) + lut_lane_addr;
-                                    asm("ld.shared.f32 %0, [%1];" : "=f"(wgt) : "r"(addr));
-                                    ws[i] = __fadd_rn(ws[i], wgt);
-                                    ps[i] = __fadd_rn(ps[i], __fmul_rn(wgt, pixv[g + i]));
-                                }
-                            }
-                        }
-                    }
-                    *reinterpret_cast<float4 *>(acc_ws + oy * kTileW + lane * 4) = make_float4(ws[0], ws[1], ws[2], ws[3]);
-                    *reinterpret_cast<float4 *>(acc_ps + oy * kTileW + lane * 4) = make_float4(ps[0], ps[1], ps[2], ps[3]);
-                }
-#pragma unroll
-                for (int r = 0; r + 1 < NH; r++)
-#pragma unroll
-                    for (int j = 0; j < NWB; j++) delay[r][j] = delay[r + 1][j];
-#pragma unroll
-                for (int j = 0; j < NWB; j++) delay[NH - 1][j] = wbv[j];
-            }
-        }
-    }
-}
-
-template <int NH, int TH, int NW>
-__global__ void __launch_bounds__(NW * 32, 1) nlmeans_fast16_kernel(const __grid_constant__ FusedParams fp)
-{
-    if (*fp.range_flag != 0u) return;               // out-of-range samples seen: the integer kernel takes over
-    constexpr int kThreads = NW * 32;
-    int pl = 0;
-    while (pl + 1 < fp.nplanes && (int)blockIdx.x >= fp.first_tile[pl + 1]) pl++;
-    const KernelParams &p = fp.k[pl];
-    const CUtensorMap *maps = fp.maps[pl];
-    const int tile = (int)blockIdx.x - fp.first_tile[pl];
-    using L = Fast16Layout<TH>;
-    extern __shared__ __align__(128) uint8_t smem[];
-    uint16_t *cur = reinterpret_cast<uint16_t *>(smem + L::kOffCur);
-    uint16_t *cmp = reinterpret_cast<uint16_t *>(smem + L::kOffCmp);
-    float *acc_ws = reinterpret_cast<float *>(smem + L::kOffWs);
-    float *acc_ps = reinterpret_cast<float *>(smem + L::kOffPs);
-    float *lut    = reinterpret_cast<float *>(smem + L::kOffLut);
-    uint64_t *bar = reinterpret_cast<uint64_t *>(smem + L::kOffBar);
-
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int X0 = (tile % fp.tiles_x[pl]) * kTileW, Y0 = (tile / fp.tiles_x[pl]) * TH;
-    const int gx = X0 + kBorder - kHaloX, gy = Y0 + kBorder - kHalo;
-
-    if (tid == 0)
-    {
-        mbar_init(bar, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    uint32_t phase = 0;
-    if (tid == 0)
-    {
-        mbar_expect_tx(bar, L::kTileBytes);
-        tma_load_2d(cur, &maps[0], gx, gy, bar);
-    }
-    for (int i = tid; i < kLutEntries * 32; i += kThreads)
-    {
-        const int e = i >> 5;
-        lut[i] = e < HBCU_NLMEANS_EXPSIZE ? p.exptable[e] : 0.f;
-    }
-    for (int i = tid; i < TH * kTileW; i += kThreads)
-    {
-        acc_ws[i] = 0.f;
-        acc_ps[i] = 0.f;
-    }
-    mbar_wait(bar, phase);
-    phase ^= 1;
-    __syncthreads();
-
-    const int seg_y0 = warp * (TH / NW);
-    const float wscale = p.wfact * 0.0078125f;                         // wfact / 128, exact
-    const uint32_t lut_lane_addr = smem_u32(lut) + (uint32_t)lane * 4u - (0x47800000u << 7);
-    for (int f = 0; f < p.nf; f++)
-    {
-        const uint16_t *B = cur;
-        if (f > 0)
-        {
-            __syncthreads();
-            if (tid == 0)
-            {
-                fence_proxy_async();
-                mbar_expect_tx(bar, L::kTileBytes);
-                tma_load_2d(cmp, &maps[f], gx, gy, bar);
-            }
-            mbar_wait(bar, phase);
-            phase ^= 1;
-            B = cmp;
-        }
-        const uint2 *cq = reinterpret_cast<const uint2 *>(cur), *bq = reinterpret_cast<const uint2 *>(B);
-        for (int dy = -p.r_half; dy <= p.r_half; dy++)
-        {
-            for (int dx0 = -p.r_half; dx0 <= p.r_half; dx0 += kGroup)
-            {
-                const int ng = min(kGroup, p.r_half - dx0 + 1);
-                const int origin_g = (f == 0 && dy == 0 && dx0 <= 0 && dx0 + ng > 0) ? -dx0 : -1;
-                if (origin_g >= 0)
-                    nlm_group_fast16<NH, TH, NW, true>(cq, bq, acc_ws, acc_ps, lut_lane_addr, wscale, p.origin_tune, seg_y0, lane, dy, dx0, ng, origin_g);
-                else
-                    nlm_group_fast16<NH, TH, NW, false>(cq, bq, acc_ws, acc_ps, lut_lane_addr, wscale, p.origin_tune, seg_y0, lane, dy, dx0, ng, -1);
-            }
-        }
-    }
-
-    const int x = lane * 4;
-    uint16_t *dst = reinterpret_cast<uint16_t *>(p.dst);
-    for (int r = 0; r < TH / NW; r++)
-    {
-        const int oy = seg_y0 + r;
-        const int y = Y0 + oy;
-        if (y >= p.h) break;
-        const float4 ws4 = *reinterpret_cast<const float4 *>(acc_ws + oy * kTileW + x);
-        const float4 ps4 = *reinterpret_cast<const float4 *>(acc_ps + oy * kTileW + x);
-        const float ws[4] = { ws4.x, ws4.y, ws4.z, ws4.w };
-        const float ps[4] = { ps4.x, ps4.y, ps4.z, ps4.w };
-        uint16_t o[4];
-#pragma unroll
-        for (int i = 0; i < 4; i++)
-            o[i] = finish_pixel<uint16_t>(ws[i], ps[i], cur[(oy + kHalo) * kTilePW + x + kHaloX + i]);
-        uint16_t *drow = dst + (size_t)y * p.dpitch + X0 + x;
-        if (X0 + x + 3 < p.w)
-            *reinterpret_cast<ushort4 *>(drow) = make_ushort4(o[0], o[1], o[2], o[3]);
-        else
-        {
-#pragma unroll
-            for (int i = 0; i < 4; i++)
-                if (X0 + x + i < p.w) drow[i] = o[i];
-        }
-    }
-}
-
 // ---------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------
@@ -1489,13 +739,11 @@ struct hbcu_nlmeans_s
     std::vector<CUtensorMap> maps;        // [slot*3+plane] TMA descriptors of the bordered planes
     std::vector<CUtensorMap> maps3;       // same planes, box height of the v3 8-bit kernel's tile
     std::vector<CUtensorMap> maps3_pre;   // the prefiltered planes (pre_mem), same box
-    int v3_nw, v3_rs, v3_tmem;            // v3 kernel shape (warps, rows per warp, accumulators in tensor memory); v3_nw == 0: off
     float *d_exptable;                    // 3 x 128
-    unsigned *d_range_flag;               // sticky: a 16-bit plane held a sample above kFast16Max (see nlmeans_fast16_kernel)
-    cudaStream_t s_h2d, s_pad, s_compute, s_d2h;   // s_compute = s_comp[frame index & (n_comp - 1)] of the launch being queued
+    unsigned *d_range_flag;               // sticky: a 16-bit plane held a sample above kMax10Bit (see nlmeans_v3w_kernel)
+    cudaStream_t s_h2d, s_pad, s_compute, s_d2h;   // s_compute = s_comp[frame index & 1] of the launch being queued
     cudaStream_t s_comp[2];               // consecutive frames alternate between two compute streams: the next frame's CTAs
                                           // fill the SMs the previous launch's last partial wave leaves idle
-    int n_comp;
     cudaEvent_t ev_join[2];
     std::vector<cudaEvent_t> ev_h2d;      // per ring slot: raw planes have arrived (H2D done), border kernels may start
     std::vector<cudaEvent_t> ev_upload;   // per ring slot: bordered planes ready
@@ -1522,311 +770,72 @@ struct hbcu_nlmeans_s
 
 namespace {
 
-template <typename PIX, int NH, int TH>
-int launch_tiled(const TiledParams &kp, cudaStream_t st)
-{
-    using L = TileLayout<PIX, TH>;
-    // function attributes live in the device's context: one flag per device (a second GPU would otherwise launch with
-    // the default 48 KB limit -- 'invalid argument'; found by the first run of devices=0,1)
-    static bool configured_on[kMaxDevices] = {};
-    int dev_ = 0;
-    HBCU_CHECK(cudaGetDevice(&dev_));
-    bool &configured = configured_on[dev_ & (kMaxDevices - 1)];
-    if (!configured)
-    {
-        HBCU_CHECK(cudaFuncSetAttribute(nlmeans_tiled_kernel<PIX, NH, TH>,
-                                        cudaFuncAttributeMaxDynamicSharedMemorySize, L::kTotal));
-        configured = true;
-    }
-    dim3 grid((kp.k.w + kTileW - 1) / kTileW, (kp.k.h + TH - 1) / TH);
-    nlmeans_tiled_kernel<PIX, NH, TH><<<grid, kThreads, L::kTotal, st>>>(kp);
-    hbcu::count_launch();
-    return 0;
-}
-
-template <int NH, int TH, int NW, bool DP4A>
-int launch_fast8(FusedParams &fp, cudaStream_t st)
-{
-    using L = FastLayout<TH>;
-    // function attributes live in the device's context: one flag per device (a second GPU would otherwise launch with
-    // the default 48 KB limit -- 'invalid argument'; found by the first run of devices=0,1)
-    static bool configured_on[kMaxDevices] = {};
-    int dev_ = 0;
-    HBCU_CHECK(cudaGetDevice(&dev_));
-    bool &configured = configured_on[dev_ & (kMaxDevices - 1)];
-    if (!configured)
-    {
-        HBCU_CHECK(cudaFuncSetAttribute(nlmeans_fast8_kernel<NH, TH, NW, DP4A>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::kTotal));
-        configured = true;
-    }
-    int total = 0;
-    for (int i = 0; i < fp.nplanes; i++)
-    {
-        fp.first_tile[i] = total;
-        fp.tiles_x[i] = (fp.k[i].w + kTileW - 1) / kTileW;
-        total += fp.tiles_x[i] * ((fp.k[i].h + TH - 1) / TH);
-    }
-    fp.first_tile[fp.nplanes] = total;
-    nlmeans_fast8_kernel<NH, TH, NW, DP4A><<<total, NW * 32, L::kTotal, st>>>(fp);
-    hbcu::count_launch();
-    return 0;
-}
-
-template <int NH, int TH, int NW>
-int launch_fast16(FusedParams &fp, cudaStream_t st)
-{
-    using L = Fast16Layout<TH>;
-    // function attributes live in the device's context: one flag per device (a second GPU would otherwise launch with
-    // the default 48 KB limit -- 'invalid argument'; found by the first run of devices=0,1)
-    static bool configured_on[kMaxDevices] = {};
-    int dev_ = 0;
-    HBCU_CHECK(cudaGetDevice(&dev_));
-    bool &configured = configured_on[dev_ & (kMaxDevices - 1)];
-    if (!configured)
-    {
-        HBCU_CHECK(cudaFuncSetAttribute(nlmeans_fast16_kernel<NH, TH, NW>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::kTotal));
-        configured = true;
-    }
-    int total = 0;
-    for (int i = 0; i < fp.nplanes; i++)
-    {
-        fp.first_tile[i] = total;
-        fp.tiles_x[i] = (fp.k[i].w + kTileW - 1) / kTileW;
-        total += fp.tiles_x[i] * ((fp.k[i].h + TH - 1) / TH);
-    }
-    fp.first_tile[fp.nplanes] = total;
-    nlmeans_fast16_kernel<NH, TH, NW><<<total, NW * 32, L::kTotal, st>>>(fp);
-    hbcu::count_launch();
-    return 0;
-}
-
-// 16-bit tiles are 128 x 96 for every kernel (they share the tensor maps): 8 warps x 12 rows
+// Tile heights of the tiled kernel: 128 x 144 for 8-bit planes, 128 x 96 for 16-bit planes (8 warps; the tensor maps
+// `maps` are encoded for this box).
+constexpr int kTH8 = 144;
 constexpr int kTH16 = 96;
 
-int launch_fast16_nh(FusedParams &kp, cudaStream_t st)
+// v3 shapes (warps x rows per warp), measured on B200 (profiles/r02b_v3_shape_sweep.txt): 12 x 18 beat 12 x 21, 8 x 28 and
+// 12 x 12 with shared-memory accumulators.  Patch 9 takes 8 warps x 27 rows: its 9-row history does not fit 168 registers.
+// Both tiles are 216 rows high, so one tensor map box (`maps3`, `maps3_pre`) serves every v3 kernel.
+using V3L   = V3Layout<12, 18, 2>;          // 8-bit, two compare buffers
+using V3L9  = V3Layout<8, 27, 2>;           // 8-bit, patch 9
+using V3LP  = V3Layout<12, 18, 1, 1, true>; // 8-bit, prefiltered planes: one compare buffer pair
+using V3LW  = V3Layout<12, 18, 1, 2>;       // 16-bit: one compare buffer (two 74 KB tiles)
+constexpr int kV3BoxRows = V3L::kBoxRows;
+static_assert(V3L9::kBoxRows == kV3BoxRows && V3LP::kBoxRows == kV3BoxRows && V3LW::kBoxRows == kV3BoxRows &&
+              V3L9::kTH == V3L::kTH, "every v3 kernel loads the same TMA box");
+
+enum class Kern { GENERIC, TILED, V3, V3W, V3_PRE };
+
+// One kernel instantiation: entry point, block size, dynamic shared memory, tile height.
+struct Inst { const void *fn; int threads, smem, th; };
+
+// The instantiation kernel `k` runs for a plane of `bps` bytes per sample and patch half-width nh; fn == nullptr where
+// there is none.
+Inst instance(Kern k, int bps, int nh)
 {
-    switch (kp.k[0].n_half)
-    {
-        case 1: return launch_fast16<1, kTH16, 8>(kp, st);
-        case 2: return launch_fast16<2, kTH16, 8>(kp, st);
-        case 3: return launch_fast16<3, kTH16, 8>(kp, st);
-        default: return 1;
-    }
-}
-
-// 8-bit tiles are 128 x 144: 12 warps x 12 rows for patch <= 7 (measured 7 % faster than 8 warps x 16 rows:
-// more warps hide the dependent-issue latency better than the extra warm-up rows cost), 8 warps x 18 rows
-// for patch 9 whose register footprint does not allow 384 threads.
-constexpr int kTH8 = 144;
-
-int g_ssd_variant = 1;     // 1: packed-byte VABSDIFF4 + IDP4A patch-row sums (measured 7 % faster), 0: fp32 prefix sums (FFMA);
-                           // HBCU_NLMEANS_SSD selects (test/tuning hook: both are exact, tests run both)
-
-template <int NH, int NW, int RS, bool TMEM, int NBUF>
-int launch_v3(FusedParams &fp, cudaStream_t st)
-{
-    using L = V3Layout<NW, RS, TMEM, NBUF>;
-    // function attributes live in the device's context: one flag per device (a second GPU would otherwise launch with
-    // the default 48 KB limit -- 'invalid argument'; found by the first run of devices=0,1)
-    static bool configured_on[kMaxDevices] = {};
-    int dev_ = 0;
-    HBCU_CHECK(cudaGetDevice(&dev_));
-    bool &configured = configured_on[dev_ & (kMaxDevices - 1)];
-    if (!configured)
-    {
-        HBCU_CHECK(cudaFuncSetAttribute(nlmeans_v3_kernel<NH, NW, RS, TMEM, NBUF>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::kTotal));
-        configured = true;
-    }
-    int total = 0;
-    for (int i = 0; i < fp.nplanes; i++)
-    {
-        fp.first_tile[i] = total;
-        fp.tiles_x[i] = (fp.k[i].w + kTileW - 1) / kTileW;
-        total += fp.tiles_x[i] * ((fp.k[i].h + L::kTH - 1) / L::kTH);
-    }
-    fp.first_tile[fp.nplanes] = total;
-    nlmeans_v3_kernel<NH, NW, RS, TMEM, NBUF><<<total, NW * 32, L::kTotal, st>>>(fp);
-    hbcu::count_launch();
-    return 0;
-}
-
-template <int NH, int NW, int RS, bool TMEM, int NBUF>
-int launch_v3w(FusedParams &fp, cudaStream_t st)
-{
-    using L = V3Layout<NW, RS, TMEM, NBUF, 2>;
-    // function attributes live in the device's context: one flag per device (a second GPU would otherwise launch with
-    // the default 48 KB limit -- 'invalid argument'; found by the first run of devices=0,1)
-    static bool configured_on[kMaxDevices] = {};
-    int dev_ = 0;
-    HBCU_CHECK(cudaGetDevice(&dev_));
-    bool &configured = configured_on[dev_ & (kMaxDevices - 1)];
-    if (!configured)
-    {
-        HBCU_CHECK(cudaFuncSetAttribute(nlmeans_v3w_kernel<NH, NW, RS, TMEM, NBUF>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::kTotal));
-        configured = true;
-    }
-    int total = 0;
-    for (int i = 0; i < fp.nplanes; i++)
-    {
-        fp.first_tile[i] = total;
-        fp.tiles_x[i] = (fp.k[i].w + kTileW - 1) / kTileW;
-        total += fp.tiles_x[i] * ((fp.k[i].h + L::kTH - 1) / L::kTH);
-    }
-    fp.first_tile[fp.nplanes] = total;
-    nlmeans_v3w_kernel<NH, NW, RS, TMEM, NBUF><<<total, NW * 32, L::kTotal, st>>>(fp);
-    hbcu::count_launch();
-    return 0;
-}
-
-// prefilter variant (patch distances from the pre-denoised planes): one plane per launch, 12 x 18, one compare buffer pair
-template <int NH>
-int launch_v3_pre(FusedParams &fp, cudaStream_t st)
-{
-    constexpr int NW = 12, RS = 18;
-    using L = V3Layout<NW, RS, true, 1, 1, true>;
-    // function attributes live in the device's context: one flag per device (a second GPU would otherwise launch with
-    // the default 48 KB limit -- 'invalid argument'; found by the first run of devices=0,1)
-    static bool configured_on[kMaxDevices] = {};
-    int dev_ = 0;
-    HBCU_CHECK(cudaGetDevice(&dev_));
-    bool &configured = configured_on[dev_ & (kMaxDevices - 1)];
-    if (!configured)
-    {
-        HBCU_CHECK(cudaFuncSetAttribute(nlmeans_v3_kernel<NH, NW, RS, true, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::kTotal));
-        configured = true;
-    }
-    int total = 0;
-    for (int i = 0; i < fp.nplanes; i++)
-    {
-        fp.first_tile[i] = total;
-        fp.tiles_x[i] = (fp.k[i].w + kTileW - 1) / kTileW;
-        total += fp.tiles_x[i] * ((fp.k[i].h + L::kTH - 1) / L::kTH);
-    }
-    fp.first_tile[fp.nplanes] = total;
-    nlmeans_v3_kernel<NH, NW, RS, true, 1, true><<<total, NW * 32, L::kTotal, st>>>(fp);
-    hbcu::count_launch();
-    return 0;
-}
-
-// v3 shapes built into the library: {warps, rows per warp, accumulators in tensor memory}.  Patch 9 (NH = 4) needs
-// 8 warps (its 9-row history does not fit 168 registers).
-struct V3Shape { int nw, rs, tmem; };
-constexpr V3Shape kV3Default = { 12, 18, 1 };      // measured on B200 (profiles/r02b_v3_shape_sweep.txt): 12x18 > 12x21 > 8x28 > 12x12 (shared-memory accumulators)
-
-// rows of one TMA box of the v3 tile: V3Layout::kBoxRows restated for a run-time shape (the kernel's expect-tx byte
-// count and the tensor map must agree)
-int v3_box_rows(int nw, int rs)
-{
-    const int rows = nw * rs + 2 * kHalo, loads = rows > 256 ? 2 : 1;
-    return ((rows + loads - 1) / loads + 3) / 4 * 4;
-}
-
-bool v3_shape_ok(int nw, int rs, int tmem, int n_half)
-{
-    if (n_half == 4) return nw == 8 && rs == 27 && tmem == 1;
-    if (nw == 12 && rs == 18 && tmem == 1) return true;
-#ifdef HBCU_V3_SWEEP_SHAPES
-    if (nw == 12 && rs == 12 && tmem == 0) return true;
-    if (n_half == 3) return tmem == 1 && ((nw == 12 && rs == 21) || (nw == 8 && rs == 28));
-#endif
-    return false;
-}
-
-// the shape a plane with patch half-width n_half runs in, given the handle's shape (whose TMA box its tensor maps
-// were encoded for): patch 9 takes the 8-warp shape with the same tile height as 12 x 18
-bool v3_pick(const hbcu_nlmeans_s *h, int n_half, V3Shape *out)
-{
-    if (h->v3_nw <= 0) return false;
-    V3Shape s = { h->v3_nw, h->v3_rs, h->v3_tmem };
-    if (n_half == 4)
-    {
-        s = V3Shape{ 8, 27, 1 };
-        if (v3_box_rows(s.nw, s.rs) != v3_box_rows(h->v3_nw, h->v3_rs) || s.nw * s.rs != h->v3_nw * h->v3_rs) return false;
-    }
-    if (!v3_shape_ok(s.nw, s.rs, s.tmem, n_half)) return false;
-    *out = s;
-    return true;
-}
-
-int launch_v3_nh(int nw, int rs, int tmem, FusedParams &fp, cudaStream_t st)
-{
-    const int nh = fp.k[0].n_half;
-    // every displacement row of this range must decompose into group shapes the kernels were built with
-    for (int pl = 0; pl < fp.nplanes; pl++)
-        for (int dx0 = -fp.k[pl].r_half; dx0 <= fp.k[pl].r_half; dx0 += kGroup)
+    if (k == Kern::V3 && bps == 1)
+        switch (nh)
         {
-            const int ng = std::min(kGroup, fp.k[pl].r_half - dx0 + 1);
-            if (!v3_group_known(ng, (12 + dx0) & 3, kOrgNone)) return 1;
-            if (dx0 <= 0 && dx0 + ng > 0 && !v3_group_known(ng, (12 + dx0) & 3, -dx0)) return 1;
+            case 1: return { (const void *)nlmeans_v3_kernel<1, 12, 18, 2>, 12 * 32, V3L::kTotal, V3L::kTH };
+            case 2: return { (const void *)nlmeans_v3_kernel<2, 12, 18, 2>, 12 * 32, V3L::kTotal, V3L::kTH };
+            case 3: return { (const void *)nlmeans_v3_kernel<3, 12, 18, 2>, 12 * 32, V3L::kTotal, V3L::kTH };
+            case 4: return { (const void *)nlmeans_v3_kernel<4, 8, 27, 2>, 8 * 32, V3L9::kTotal, V3L9::kTH };
         }
-#define V3CASE(NH_, NW_, RS_, TM_, NB_) if (nh == NH_ && nw == NW_ && rs == RS_ && tmem == TM_) return launch_v3<NH_, NW_, RS_, TM_ != 0, NB_>(fp, st)
-    V3CASE(1, 12, 18, 1, 2); V3CASE(2, 12, 18, 1, 2); V3CASE(3, 12, 18, 1, 2);
-    V3CASE(4, 8, 27, 1, 2);
-#ifdef HBCU_V3_SWEEP_SHAPES
-    // the other shapes of profiles/r02b_v3_shape_sweep.txt (shared-memory accumulators, 252-row tile, 8 warps): built only
-    // with -DHBCU_V3_SWEEP_SHAPES, they cost minutes of compile time and lost the sweep
-    V3CASE(1, 12, 12, 0, 1); V3CASE(2, 12, 12, 0, 1); V3CASE(3, 12, 12, 0, 1);
-    V3CASE(3, 12, 21, 1, 2); V3CASE(3, 8, 28, 1, 2);
-#endif
-#undef V3CASE
-    return 1;
-}
-
-// 16-bit planes: one shape (12 warps x 18 rows, accumulators in tensor memory, one compare buffer: two 74 KB tiles)
-constexpr V3Shape kV3wShape = { 12, 18, 1 };
-
-int launch_v3w_nh(FusedParams &fp, cudaStream_t st)
-{
-    for (int pl = 0; pl < fp.nplanes; pl++)
-        for (int dx0 = -fp.k[pl].r_half; dx0 <= fp.k[pl].r_half; dx0 += kGroup)
+    if (k == Kern::V3_PRE && bps == 1)
+        switch (nh)
         {
-            const int ng = std::min(kGroup, fp.k[pl].r_half - dx0 + 1);
-            if (!v3_group_known(ng, (12 + dx0) & 3, kOrgNone)) return 1;
-            if (dx0 <= 0 && dx0 + ng > 0 && !v3_group_known(ng, (12 + dx0) & 3, -dx0)) return 1;
+            case 1: return { (const void *)nlmeans_v3_kernel<1, 12, 18, 1, true>, 12 * 32, V3LP::kTotal, V3LP::kTH };
+            case 2: return { (const void *)nlmeans_v3_kernel<2, 12, 18, 1, true>, 12 * 32, V3LP::kTotal, V3LP::kTH };
+            case 3: return { (const void *)nlmeans_v3_kernel<3, 12, 18, 1, true>, 12 * 32, V3LP::kTotal, V3LP::kTH };
         }
-    switch (fp.k[0].n_half)
-    {
-        case 1: return launch_v3w<1, kV3wShape.nw, kV3wShape.rs, true, 1>(fp, st);
-        case 2: return launch_v3w<2, kV3wShape.nw, kV3wShape.rs, true, 1>(fp, st);
-        case 3: return launch_v3w<3, kV3wShape.nw, kV3wShape.rs, true, 1>(fp, st);
-        default: return 1;
-    }
-}
-
-int launch_fast8_nh(FusedParams &kp, cudaStream_t st)
-{
-    if (g_ssd_variant == 1)
-    {
-        switch (kp.k[0].n_half)
+    if (k == Kern::V3W && bps == 2)
+        switch (nh)
         {
-            case 1: return launch_fast8<1, kTH8, 12, true>(kp, st);
-            case 2: return launch_fast8<2, kTH8, 12, true>(kp, st);
-            case 3: return launch_fast8<3, kTH8, 12, true>(kp, st);
-            case 4: return launch_fast8<4, kTH8, 8, true>(kp, st);
-            default: return 1;
+            case 1: return { (const void *)nlmeans_v3w_kernel<1, 12, 18, 1>, 12 * 32, V3LW::kTotal, V3LW::kTH };
+            case 2: return { (const void *)nlmeans_v3w_kernel<2, 12, 18, 1>, 12 * 32, V3LW::kTotal, V3LW::kTH };
+            case 3: return { (const void *)nlmeans_v3w_kernel<3, 12, 18, 1>, 12 * 32, V3LW::kTotal, V3LW::kTH };
         }
-    }
-    switch (kp.k[0].n_half)
-    {
-        case 1: return launch_fast8<1, kTH8, 12, false>(kp, st);
-        case 2: return launch_fast8<2, kTH8, 12, false>(kp, st);
-        case 3: return launch_fast8<3, kTH8, 12, false>(kp, st);
-        case 4: return launch_fast8<4, kTH8, 8, false>(kp, st);
-        default: return 1;
-    }
-}
-
-template <typename PIX, int TH>
-int launch_tiled_nh(const TiledParams &kp, cudaStream_t st)
-{
-    switch (kp.k.n_half)
-    {
-        case 1: return launch_tiled<PIX, 1, TH>(kp, st);
-        case 2: return launch_tiled<PIX, 2, TH>(kp, st);
-        case 3: return launch_tiled<PIX, 3, TH>(kp, st);
-        case 4: return launch_tiled<PIX, 4, TH>(kp, st);
-        default: return 1;
-    }
+    using T8 = TileLayout<uint8_t, kTH8>;
+    using T16 = TileLayout<uint16_t, kTH16>;
+    if (k == Kern::TILED && bps == 1)
+        switch (nh)
+        {
+            case 1: return { (const void *)nlmeans_tiled_kernel<uint8_t, 1, kTH8>, kThreads, T8::kTotal, kTH8 };
+            case 2: return { (const void *)nlmeans_tiled_kernel<uint8_t, 2, kTH8>, kThreads, T8::kTotal, kTH8 };
+            case 3: return { (const void *)nlmeans_tiled_kernel<uint8_t, 3, kTH8>, kThreads, T8::kTotal, kTH8 };
+            case 4: return { (const void *)nlmeans_tiled_kernel<uint8_t, 4, kTH8>, kThreads, T8::kTotal, kTH8 };
+        }
+    if (k == Kern::TILED && bps == 2)
+        switch (nh)
+        {
+            case 1: return { (const void *)nlmeans_tiled_kernel<uint16_t, 1, kTH16>, kThreads, T16::kTotal, kTH16 };
+            case 2: return { (const void *)nlmeans_tiled_kernel<uint16_t, 2, kTH16>, kThreads, T16::kTotal, kTH16 };
+            case 3: return { (const void *)nlmeans_tiled_kernel<uint16_t, 3, kTH16>, kThreads, T16::kTotal, kTH16 };
+            case 4: return { (const void *)nlmeans_tiled_kernel<uint16_t, 4, kTH16>, kThreads, T16::kTotal, kTH16 };
+        }
+    return { nullptr, 0, 0, 0 };
 }
 
 bool tiled_supported(const KernelParams &kp)
@@ -1834,89 +843,96 @@ bool tiled_supported(const KernelParams &kp)
     return !kp.use_pre && kp.n_half >= 1 && kp.n_half <= 4 && kp.n_half + kp.r_half <= kHalo && kp.nf <= kMaxTiledFrames;
 }
 
-bool fast8_ok(const hbcu_nlmeans_s *h, const KernelParams &kp)
+// every displacement row of the plane's range decomposes into group shapes the v3 kernels were built with (all ranges
+// 3 .. 15; range 1 does not)
+bool v3_groups_known(const KernelParams &kp)
 {
-    // fp32-exact fast kernel: 8-bit planes, halo fits, the saturating table trick is valid (wfact < 0.99)
-    return h->bps == 1 && h->impl != 1 && h->impl != 3 && tiled_supported(kp) && kp.wfact < 0.99f && kp.wfact > 1e-5f;
+    for (int dx0 = -kp.r_half; dx0 <= kp.r_half; dx0 += kGroup)
+    {
+        const int ng = std::min(kGroup, kp.r_half - dx0 + 1), ob = (12 + dx0) & 3;
+        if (!v3_group_known(ng, ob, kOrgNone)) return false;
+        if (dx0 <= 0 && dx0 + ng > 0 && !v3_group_known(ng, ob, -dx0)) return false;
+    }
+    return true;
 }
 
-bool fast16_ok(const hbcu_nlmeans_s *h, const KernelParams &kp)
+// The kernel a plane runs (hbcu_nlmeans_set_impl): impl 1 the generic kernel, impl 3 the integer tiled kernel where it
+// fits; impl 0 and 2 a v3 kernel where its conditions hold, else the tiled kernel, else the generic one (which impl 2
+// refuses, in run_filter).
+Kern pick_kernel(const hbcu_nlmeans_s *h, const KernelParams &kp)
 {
-    // fp32-exact fast kernel for 9/10-bit planes: patch <= 7, same table trick
-    return h->bps == 2 && h->cfg.depth <= 10 && h->impl != 1 && h->impl != 3 && tiled_supported(kp) && kp.n_half <= 3 &&
-           kp.wfact < 0.99f && kp.wfact > 1e-5f;
+    const bool tiled = tiled_supported(kp);
+    if (h->impl == 1) return Kern::GENERIC;
+    if (h->impl == 3) return tiled ? Kern::TILED : Kern::GENERIC;
+    const bool v3 = kp.wfact < 0.99f && kp.wfact > 1e-5f && v3_groups_known(kp);    // the table trick, the group shapes
+    if (v3 && kp.use_pre && h->bps == 1 && kp.n_half >= 1 && kp.n_half <= 3 && kp.n_half + kp.r_half <= kHalo &&
+        kp.nf <= kMaxTiledFrames)
+        return Kern::V3_PRE;
+    if (v3 && tiled && h->bps == 1) return Kern::V3;
+    if (v3 && tiled && h->bps == 2 && h->cfg.depth <= 10 && kp.n_half <= 3) return Kern::V3W;
+    return tiled ? Kern::TILED : Kern::GENERIC;
 }
 
-int launch_plane(hbcu_nlmeans_s *h, const KernelParams &kp, const int *slots, int plane, const unsigned *only_if_flag = nullptr)
+// The integer tiled kernel on one plane.  only_if_flag: run only if *only_if_flag != 0 (the stand-in behind a v3w launch).
+int launch_tiled(hbcu_nlmeans_s *h, const KernelParams &kp, const int *slots, int plane, const unsigned *only_if_flag)
 {
-    // prefilter modes on 8-bit planes: the v3 kernel's prefilter variant (VERDICT r1 missing 5: these settings used to fall
-    // to the one-thread-per-pixel generic kernel); same validity conditions as the plain fast kernel
-    if (kp.use_pre && only_if_flag == nullptr && h->bps == 1 && h->impl == 0 && h->v3_nw == 12 && h->v3_rs == 18 && h->v3_tmem == 1 &&
-        kp.n_half >= 1 && kp.n_half <= 3 && kp.n_half + kp.r_half <= kHalo && kp.nf <= kMaxTiledFrames && kp.wfact < 0.99f && kp.wfact > 1e-5f)
-    {
-        bool known = true;
-        for (int dx0 = -kp.r_half; dx0 <= kp.r_half; dx0 += kGroup)
-        {
-            const int ng = std::min(kGroup, kp.r_half - dx0 + 1);
-            known = known && v3_group_known(ng, (12 + dx0) & 3, kOrgNone) && (!(dx0 <= 0 && dx0 + ng > 0) || v3_group_known(ng, (12 + dx0) & 3, -dx0));
-        }
-        if (known)
-        {
-            FusedParams fp;
-            fp.nplanes = 1;
-            fp.range_flag = nullptr;
-            fp.k[0] = kp;
-            for (int f = 0; f < kp.nf; f++)
-            {
-                fp.maps[0][f] = h->maps3[slots[f] * 3 + plane];
-                fp.maps_pre[0][f] = h->maps3_pre[slots[f] * 3 + plane];
-            }
-            const int rc = kp.n_half == 1 ? launch_v3_pre<1>(fp, h->s_compute) : kp.n_half == 2 ? launch_v3_pre<2>(fp, h->s_compute) : launch_v3_pre<3>(fp, h->s_compute);
-            if (rc != 0) return rc;
-            HBCU_CHECK(cudaGetLastError());
-            return 0;
-        }
-    }
-    const bool want_tiled = h->impl != 1 && tiled_supported(kp);
-    if (h->impl == 2 && !want_tiled)
-    {
-        set_error("nlmeans: tiled kernel does not support n=%d r=%d", 2 * kp.n_half + 1, 2 * kp.r_half + 1);
-        return -1;
-    }
-    if (want_tiled)
-    {
-        TiledParams tp;
-        tp.k = kp;
-        tp.only_if_flag = only_if_flag;
-        for (int f = 0; f < kp.nf; f++) tp.maps[f] = h->maps[slots[f] * 3 + plane];
-        // impl 0/2: fp32-exact fast kernel for 8-bit planes when the table trick is valid; impl 3: integer tiled kernel
-        const bool fast_ok = fast8_ok(h, kp);
-        int rc;
-        if (fast_ok && h->impl != 3)
-        {
-            FusedParams fp;
-            fp.nplanes = 1;
-            fp.range_flag = nullptr;
-            fp.k[0] = kp;
-            V3Shape vs;
-            const bool v3 = v3_pick(h, kp.n_half, &vs);
-            for (int f = 0; f < kp.nf; f++) fp.maps[0][f] = v3 ? h->maps3[slots[f] * 3 + plane] : tp.maps[f];
-            rc = v3 ? launch_v3_nh(vs.nw, vs.rs, vs.tmem, fp, h->s_compute) : launch_fast8_nh(fp, h->s_compute);
-        }
-        else
-            rc = h->bps == 1 ? launch_tiled_nh<uint8_t, kTH8>(tp, h->s_compute) : launch_tiled_nh<uint16_t, kTH16>(tp, h->s_compute);
-        if (rc < 0) return rc;
-        if (rc == 0)
-        {
-            HBCU_CHECK(cudaGetLastError());
-            return 0;
-        }
-    }
-    dim3 blk(32, 8), grid((kp.w + 31) / 32, (kp.h + 7) / 8);
-    if (h->bps == 1) nlmeans_generic_kernel<uint8_t><<<grid, blk, 0, h->s_compute>>>(kp);
-    else             nlmeans_generic_kernel<uint16_t><<<grid, blk, 0, h->s_compute>>>(kp);
+    TiledParams tp;
+    tp.k = kp;
+    tp.only_if_flag = only_if_flag;
+    for (int f = 0; f < kp.nf; f++) tp.maps[f] = h->maps[slots[f] * 3 + plane];
+    const Inst in = instance(Kern::TILED, h->bps, kp.n_half);
+    void *args[] = { &tp };
+    HBCU_CHECK(cudaLaunchKernel(in.fn, dim3((kp.w + kTileW - 1) / kTileW, (kp.h + in.th - 1) / in.th), dim3(in.threads), args,
+                                (size_t)in.smem, h->s_compute));
     hbcu::count_launch();
-    HBCU_CHECK(cudaGetLastError());
+    return 0;
+}
+
+// Runs kernel k on the planes pl[0 .. n).  The v3 kernels take all of them in one launch (they share n_half); the tiled
+// and generic kernels are called with one plane.
+int launch_planes(hbcu_nlmeans_s *h, Kern k, const KernelParams *kps, const int (*slots)[kMaxFrames], const int *pl, int n)
+{
+    if (k == Kern::GENERIC)
+    {
+        const KernelParams &kp = kps[pl[0]];
+        dim3 blk(32, 8), grid((kp.w + 31) / 32, (kp.h + 7) / 8);
+        if (h->bps == 1) nlmeans_generic_kernel<uint8_t><<<grid, blk, 0, h->s_compute>>>(kp);
+        else             nlmeans_generic_kernel<uint16_t><<<grid, blk, 0, h->s_compute>>>(kp);
+        hbcu::count_launch();
+        HBCU_CHECK(cudaGetLastError());
+        return 0;
+    }
+    if (k == Kern::TILED) return launch_tiled(h, kps[pl[0]], slots[pl[0]], pl[0], nullptr);
+
+    // one linear grid over the tiles of every plane: separate launches would end in one partial wave each
+    // (510 + 135 + 135 CTAs of a 4K frame on 148 SMs)
+    FusedParams fp;
+    fp.nplanes = n;
+    fp.range_flag = h->d_range_flag;
+    const Inst in = instance(k, h->bps, kps[pl[0]].n_half);
+    int total = 0;
+    for (int i = 0; i < n; i++)
+    {
+        const KernelParams &kp = kps[pl[i]];
+        fp.k[i] = kp;
+        for (int f = 0; f < kp.nf; f++)
+        {
+            fp.maps[i][f] = h->maps3[slots[pl[i]][f] * 3 + pl[i]];
+            if (k == Kern::V3_PRE) fp.maps_pre[i][f] = h->maps3_pre[slots[pl[i]][f] * 3 + pl[i]];
+        }
+        fp.first_tile[i] = total;
+        fp.tiles_x[i] = (kp.w + kTileW - 1) / kTileW;
+        total += fp.tiles_x[i] * ((kp.h + in.th - 1) / in.th);
+    }
+    fp.first_tile[n] = total;
+    void *args[] = { &fp };
+    HBCU_CHECK(cudaLaunchKernel(in.fn, dim3(total), dim3(in.threads), args, (size_t)in.smem, h->s_compute));
+    hbcu::count_launch();
+    // v3w computes nothing for a frame with samples above 10 bit (the border kernel raised the range flag); the integer
+    // kernel behind it then does the frame, and returns at once otherwise
+    if (k == Kern::V3W)
+        for (int i = 0; i < n; i++)
+            if (launch_tiled(h, kps[pl[i]], slots[pl[i]], pl[i], h->d_range_flag) != 0) return -1;
     return 0;
 }
 
@@ -1961,7 +977,7 @@ int run_filter(hbcu_nlmeans_s *h, int64_t index, int navail, int oslot, void *co
         set_error("nlmeans: navail must be >= 1");
         return -1;
     }
-    const int cs = (int)(index & (h->n_comp - 1));
+    const int cs = (int)(index & 1);
     h->s_compute = h->s_comp[cs];
     int max_nf = 1;
     for (int pl = 0; pl < 3; pl++)
@@ -2042,88 +1058,33 @@ int run_filter(hbcu_nlmeans_s *h, int64_t index, int navail, int oslot, void *co
         kp.exptable = h->d_exptable + pl * HBCU_NLMEANS_EXPSIZE;
         active[pl] = true;
     }
-    // all active planes in one launch when they can share the fast 8-bit kernel instantiation
-    bool fused = h->impl == 0 || h->impl == 2;
-    int nact = 0, nh = -1;
-    for (int pl = 0; pl < 3; pl++) nact += active[pl] ? 1 : 0;
-    for (int pl = 0; pl < 3 && fused; pl++)
+    Kern kern[3];
+    int act[3], nact = 0;
+    for (int pl = 0; pl < 3; pl++)
     {
         if (!active[pl]) continue;
-        if (!fast8_ok(h, kps[pl])) fused = false;
-        if (nh < 0) nh = kps[pl].n_half; else if (nh != kps[pl].n_half) fused = false;
+        kern[pl] = pick_kernel(h, kps[pl]);
+        if (h->impl == 2 && kern[pl] == Kern::GENERIC)
+        {
+            set_error("nlmeans: tiled kernel does not support n=%d r=%d", 2 * kps[pl].n_half + 1, 2 * kps[pl].r_half + 1);
+            return -1;
+        }
+        act[nact++] = pl;
     }
-    const int nh8 = nh;
-    bool fused16 = (h->impl == 0 || h->impl == 2) && h->bps == 2;
-    nh = -1;
-    for (int pl = 0; pl < 3 && fused16; pl++)
+    // one launch for all active planes when they picked the same v3 kernel and patch size, else one launch per plane
+    bool fused = nact > 0 && (kern[act[0]] == Kern::V3 || kern[act[0]] == Kern::V3W);
+    for (int i = 1; i < nact && fused; i++)
+        fused = kern[act[i]] == kern[act[0]] && kps[act[i]].n_half == kps[act[0]].n_half;
+    if (fused)
     {
-        if (!active[pl]) continue;
-        if (!fast16_ok(h, kps[pl])) fused16 = false;
-        if (nh < 0) nh = kps[pl].n_half; else if (nh != kps[pl].n_half) fused16 = false;
-    }
-    if (fused16 && nact > 0)
-    {
-        FusedParams fp;
-        fp.nplanes = 0;
-        fp.range_flag = h->d_range_flag;
-        for (int pl = 0; pl < 3; pl++)
-        {
-            if (!active[pl]) continue;
-            fp.k[fp.nplanes] = kps[pl];
-            for (int f = 0; f < kps[pl].nf; f++) fp.maps[fp.nplanes][f] = (h->v3_nw > 0 ? h->maps3 : h->maps)[slots[pl][f] * 3 + pl];
-            fp.nplanes++;
-        }
-        int rc16 = h->v3_nw > 0 ? launch_v3w_nh(fp, h->s_compute) : 1;
-        if (rc16 > 0)
-        {
-            // a range the v3 group shapes do not cover (or v3 switched off): the round-1 kernel on its own tensor maps
-            fp.nplanes = 0;
-            for (int pl = 0; pl < 3; pl++)
-            {
-                if (!active[pl]) continue;
-                for (int f = 0; f < kps[pl].nf; f++) fp.maps[fp.nplanes][f] = h->maps[slots[pl][f] * 3 + pl];
-                fp.nplanes++;
-            }
-            rc16 = launch_fast16_nh(fp, h->s_compute);
-        }
-        if (rc16 != 0) { set_error("nlmeans: fused 16-bit launch failed"); return -1; }
-        HBCU_CHECK(cudaGetLastError());
-        h->kernel_launches++;
-        // stand-in for frames with samples above 10 bit: returns immediately unless the border kernel raised the flag
-        const int saved_impl = h->impl;
-        h->impl = 3;
-        for (int pl = 0; pl < 3; pl++)
-        {
-            if (!active[pl]) continue;
-            if (launch_plane(h, kps[pl], slots[pl], pl, h->d_range_flag) != 0) { h->impl = saved_impl; return -1; }
-        }
-        h->impl = saved_impl;
-    }
-    else if (fused && nact > 1)
-    {
-        FusedParams fp;
-        fp.nplanes = 0;
-        fp.range_flag = nullptr;
-        V3Shape vs;
-        const bool v3 = v3_pick(h, nh8, &vs);
-        for (int pl = 0; pl < 3; pl++)
-        {
-            if (!active[pl]) continue;
-            fp.k[fp.nplanes] = kps[pl];
-            for (int f = 0; f < kps[pl].nf; f++) fp.maps[fp.nplanes][f] = (v3 ? h->maps3 : h->maps)[slots[pl][f] * 3 + pl];
-            fp.nplanes++;
-        }
-        if ((v3 ? launch_v3_nh(vs.nw, vs.rs, vs.tmem, fp, h->s_compute) : launch_fast8_nh(fp, h->s_compute)) != 0)
-        { set_error("nlmeans: fused launch failed"); return -1; }
-        HBCU_CHECK(cudaGetLastError());
+        if (launch_planes(h, kern[act[0]], kps, slots, act, nact) != 0) return -1;
         h->kernel_launches++;
     }
     else
     {
-        for (int pl = 0; pl < 3; pl++)
+        for (int i = 0; i < nact; i++)
         {
-            if (!active[pl]) continue;
-            if (launch_plane(h, kps[pl], slots[pl], pl) != 0) return -1;
+            if (launch_planes(h, kern[act[i]], kps, slots, &act[i], 1) != 0) return -1;
             h->kernel_launches++;
         }
     }
@@ -2202,21 +1163,6 @@ int hbcu_nlmeans_create(hbcu_nlmeans_t **out, const hbcu_nlmeans_config_t *cfg)
     h->bps = cfg->depth > 8 ? 2 : 1;
     h->impl = 0;
     if (const char *e = getenv("HBCU_NLMEANS_IMPL")) h->impl = atoi(e) >= 0 && atoi(e) <= 3 ? atoi(e) : 0;   // test hook
-    if (const char *e = getenv("HBCU_NLMEANS_SSD")) g_ssd_variant = atoi(e);                                  // tuning hook
-    // v3 8-bit kernel shape; HBCU_NLMEANS_V3=off | "warps,rows,tmem" (tuning hook, see v3_shape_ok)
-    h->v3_nw = kV3Default.nw; h->v3_rs = kV3Default.rs; h->v3_tmem = kV3Default.tmem;
-    if (const char *e = getenv("HBCU_NLMEANS_V3"))
-    {
-        int a = 0, b = 0, c = 0;
-        if (sscanf(e, "%d,%d,%d", &a, &b, &c) == 3 && v3_shape_ok(a, b, c, 3)) { h->v3_nw = a; h->v3_rs = b; h->v3_tmem = c; }
-        else h->v3_nw = 0;
-    }
-    if (h->bps != 1)
-    {
-        // 16-bit planes have one v3 shape (nlmeans_v3w_kernel); HBCU_NLMEANS_V3=off still selects the round-1 kernel
-        const bool off = h->v3_nw == 0;
-        h->v3_nw = off ? 0 : kV3wShape.nw; h->v3_rs = kV3wShape.rs; h->v3_tmem = kV3wShape.tmem;
-    }
     h->ring = cfg->ring_frames > 0 ? cfg->ring_frames : 8;
     h->out_slots = cfg->out_slots > 0 ? cfg->out_slots : 4;
     h->d_exptable = nullptr;
@@ -2251,11 +1197,17 @@ int hbcu_nlmeans_create(hbcu_nlmeans_t **out, const hbcu_nlmeans_config_t *cfg)
     // give the upload stream the highest priority so its CTAs are placed as soon as any SM frees up.
     int prio_lo = 0, prio_hi = 0;
     CK(cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
+    // function attributes live in the device's context: every kernel this handle can launch opts into its dynamic shared
+    // memory here, per device (a handle on a second GPU would otherwise launch with the default 48 KB limit)
+    for (Kern k : { Kern::TILED, Kern::V3, Kern::V3W, Kern::V3_PRE })
+        for (int nh = 1; nh <= 4; nh++)
+        {
+            const Inst in = instance(k, h->bps, nh);
+            if (in.fn != nullptr) CK(cudaFuncSetAttribute(in.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, in.smem));
+        }
     CK(cudaStreamCreateWithPriority(&h->s_h2d, cudaStreamNonBlocking, prio_hi));
     CK(cudaStreamCreateWithPriority(&h->s_pad, cudaStreamNonBlocking, prio_hi));    // border kernels: off the copy stream, so the
                                                                                    // copy engine never waits for an SM to free up
-    h->n_comp = 2;
-    if (const char *e = getenv("HBCU_NLMEANS_STREAMS")) h->n_comp = atoi(e) == 1 ? 1 : 2;                     // tuning hook
     CK(cudaStreamCreateWithPriority(&h->s_comp[0], cudaStreamNonBlocking, prio_lo));
     CK(cudaStreamCreateWithPriority(&h->s_comp[1], cudaStreamNonBlocking, prio_lo));
     h->s_compute = h->s_comp[0];
@@ -2316,7 +1268,7 @@ int hbcu_nlmeans_create(hbcu_nlmeans_t **out, const hbcu_nlmeans_config_t *cfg)
                 CK(cudaMemset(h->pre_mem[s * 3 + pl], 0, h->g[pl].bbytes));
             }
             h->raw_mem[s * 3 + pl] = h->raw_base[s] + h->plane_off[pl];
-            const int th = h->bps == 1 ? kTH8 : 96;
+            const int th = h->bps == 1 ? kTH8 : kTH16;
             if (hbcu::encode_tensor_map_2d(&h->maps[s * 3 + pl], h->bps, h->ring_mem[s * 3 + pl], (uint64_t)h->g[pl].bw,
                                            (uint64_t)h->g[pl].bh, (uint64_t)h->g[pl].bpitch * h->bps, kTilePW,
                                            th + 2 * kHalo) != 0)
@@ -2324,18 +1276,17 @@ int hbcu_nlmeans_create(hbcu_nlmeans_t **out, const hbcu_nlmeans_config_t *cfg)
                 hbcu_nlmeans_destroy(h);
                 return -1;
             }
-            if (h->v3_nw > 0 &&
-                hbcu::encode_tensor_map_2d(&h->maps3[s * 3 + pl], h->bps, h->ring_mem[s * 3 + pl], (uint64_t)h->g[pl].bw,
+            if (hbcu::encode_tensor_map_2d(&h->maps3[s * 3 + pl], h->bps, h->ring_mem[s * 3 + pl], (uint64_t)h->g[pl].bw,
                                            (uint64_t)h->g[pl].bh, (uint64_t)h->g[pl].bpitch * h->bps, kTilePW,
-                                           v3_box_rows(h->v3_nw, h->v3_rs)) != 0)
+                                           kV3BoxRows) != 0)
             {
                 hbcu_nlmeans_destroy(h);
                 return -1;
             }
-            if (h->v3_nw > 0 && h->has_pre[pl] &&
+            if (h->has_pre[pl] &&
                 hbcu::encode_tensor_map_2d(&h->maps3_pre[s * 3 + pl], h->bps, h->pre_mem[s * 3 + pl], (uint64_t)h->g[pl].bw,
                                            (uint64_t)h->g[pl].bh, (uint64_t)h->g[pl].bpitch * h->bps, kTilePW,
-                                           v3_box_rows(h->v3_nw, h->v3_rs)) != 0)
+                                           kV3BoxRows) != 0)
             {
                 hbcu_nlmeans_destroy(h);
                 return -1;
@@ -2779,7 +1730,7 @@ int hbcu_nlmeans_filter_frame(hbcu_nlmeans_t *h, int64_t index, int navail, hbcu
     if (h == nullptr || index < 0 || !frame_fits(h, out)) { set_error("nlmeans_filter_frame: bad argument or frame geometry"); return -1; }
     HBCU_CHECK(cudaSetDevice(h->cfg.device));
     const int oslot = (int)(index % h->out_slots);
-    cudaStream_t st = h->s_comp[index & (h->n_comp - 1)];          // the stream run_filter() will launch on
+    cudaStream_t st = h->s_comp[index & 1];          // the stream run_filter() will launch on
     if (hbcu::frame_begin_write(out, st) != 0) return -1;
     void *planes[3] = { out->plane[0], out->plane[1], out->plane[2] };
     if (run_filter(h, index, navail, oslot, planes, out->stride) != 0) return -1;

@@ -1,6 +1,6 @@
 // nlmeans_v3.cuh -- third generation of the fused 8-bit NLMeans tile kernel (included by nlmeans.cu).
 //
-// Same arithmetic contract as nlmeans_fast8_kernel (bit-identical to templates/nlmeans_template.c:593-717), same
+// Same arithmetic contract as nlmeans_tiled_kernel (bit-identical to templates/nlmeans_template.c:593-717), same
 // tiling idea (TMA tile in shared memory, a lane marches down a 4-pixel-wide column strip keeping the vertical running
 // sum of horizontal patch-row sums and its N-row history in registers).  What changed, each item from the r01 ncu
 // capture (profiles/r01g_nlmeans_fused_ncu.json: 29 thread-instructions per pixel x displacement, 68 % issue,
@@ -15,13 +15,13 @@
 //   * the three-row delay line of compare words is indexed by the unrolled row slot instead of being shifted: no MOVs;
 //   * warm-up rows are peeled: the steady-state loop has no "row >= NH" test;
 //   * the compare tile of frame 1 is in flight while frame 0 is compared with itself (second mbarrier);
-//   * accumulators (weight sum, pixel sum; 8 bytes per pixel) can live in TENSOR MEMORY (tcgen05.ld/st, 32x32b.x8:
+//   * accumulators (weight sum, pixel sum; 8 bytes per pixel) live in TENSOR MEMORY (tcgen05.ld/st, 32x32b.x8:
 //     a lane's 4 x 2 floats are 8 columns of its own TMEM lane).  That takes their 16 wavefronts per row off the
 //     shared-memory pipe and -- shared memory no longer bounds the tile -- lets a warp march 18-20 rows instead of 12:
 //     the 2*NH warm-up rows drop from 50 % to 30-33 % of the patch-row-sum work.
 #pragma once
 
-template <int NW, int RS, bool TMEM, int NBUF, int BPS = 1, bool PRE = false>
+template <int NW, int RS, int NBUF, int BPS = 1, bool PRE = false>
 struct V3Layout
 {
     static constexpr int kTH        = NW * RS;
@@ -30,7 +30,6 @@ struct V3Layout
     static constexpr int kRows      = kBoxRows * kLoads;                                 // >= kTH + 2 * kHalo; surplus rows are loaded, never used
     static constexpr int kRowBytes  = kTilePW * BPS;
     static constexpr int kTileBytes = kRows * kRowBytes;
-    static constexpr int kAccBytes  = TMEM ? 0 : kTH * kTileW * (int)sizeof(float);      // per accumulator array
     static constexpr int kLutBytes  = kLutEntries * 32 * (int)sizeof(float);
     static constexpr int kOffCur    = 0;
     static constexpr int kOffCmp    = kOffCur + kTileBytes;
@@ -38,42 +37,20 @@ struct V3Layout
     // these, pixel values from the plain tiles)
     static constexpr int kOffPre0   = kOffCmp + NBUF * kTileBytes;
     static constexpr int kOffCmpPre = kOffPre0 + (PRE ? kTileBytes : 0);
-    static constexpr int kOffWs     = kOffCmpPre + (PRE ? kTileBytes : 0);
+    static constexpr int kOffLut    = kOffCmpPre + (PRE ? kTileBytes : 0);
     static_assert(!PRE || NBUF == 1, "the prefilter variant keeps one compare buffer pair");
-    static constexpr int kOffPs     = kOffWs + kAccBytes;
-    static constexpr int kOffLut    = kOffPs + kAccBytes;
     static constexpr int kOffBar    = kOffLut + kLutBytes;                               // 1 + NBUF mbarriers, TMEM base word
     static constexpr int kUsed      = kOffBar + 64;
-    // one CTA per SM by construction (the TMEM variant allocates all 512 columns; a second resident CTA would spin)
+    // one CTA per SM by construction (the kernel allocates all 512 TMEM columns; a second resident CTA would spin)
     static constexpr int kTotal     = kUsed < 117 * 1024 ? 117 * 1024 : kUsed;
     static_assert(kBoxRows <= 256, "TMA box rows");
     static_assert((kBoxRows * kRowBytes) % 128 == 0, "TMA destination must stay 128-byte aligned");
-    static_assert(!TMEM || ((NW + 3) / 4 * RS * 8 <= 512), "accumulators must fit 512 TMEM columns per lane quarter");
+    static_assert((NW + 3) / 4 * RS * 8 <= 512, "accumulators must fit 512 TMEM columns per lane quarter");
     static_assert(kTotal <= 227 * 1024, "shared memory");
 };
 
-// accumulator rows of one warp: shared memory (float4 per lane and array) or tensor memory (8 columns per lane)
-template <bool TMEM> struct V3Acc;
-
-template <> struct V3Acc<false>
-{
-    float *ws, *ps;     // this lane's first row
-    __device__ __forceinline__ void load(int r, uint32_t (&v)[8]) const
-    {
-        const uint4 a = *reinterpret_cast<const uint4 *>(ws + r * kTileW);
-        const uint4 b = *reinterpret_cast<const uint4 *>(ps + r * kTileW);
-        v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
-    }
-    __device__ __forceinline__ void wait_load(uint32_t (&)[8]) const {}
-    __device__ __forceinline__ void store(int r, const uint32_t (&v)[8]) const
-    {
-        *reinterpret_cast<uint4 *>(ws + r * kTileW) = make_uint4(v[0], v[1], v[2], v[3]);
-        *reinterpret_cast<uint4 *>(ps + r * kTileW) = make_uint4(v[4], v[5], v[6], v[7]);
-    }
-    __device__ __forceinline__ void wait_store() const {}
-};
-
-template <> struct V3Acc<true>
+// accumulator rows of one warp in tensor memory (8 columns per lane)
+struct V3Acc
 {
     uint32_t taddr;     // lane quarter of this warp (bits 31..16) + first column of its strip
     __device__ __forceinline__ void load(int r, uint32_t (&v)[8]) const
@@ -446,11 +423,11 @@ __host__ __device__ inline bool v3_group_known(int ng, int ob, int org)
     return false;
 }
 
-template <int NH, int NW, int RS, bool TMEM, int NBUF, bool PRE = false>
+template <int NH, int NW, int RS, int NBUF, bool PRE = false>
 __global__ void __launch_bounds__(NW * 32, 1) nlmeans_v3_kernel(const __grid_constant__ FusedParams fp)
 {
     constexpr int kThreads = NW * 32;
-    using L = V3Layout<NW, RS, TMEM, NBUF, 1, PRE>;
+    using L = V3Layout<NW, RS, NBUF, 1, PRE>;
     int pl = 0;
     while (pl + 1 < fp.nplanes && (int)blockIdx.x >= fp.first_tile[pl + 1]) pl++;
     const KernelParams &p = fp.k[pl];
@@ -473,14 +450,14 @@ __global__ void __launch_bounds__(NW * 32, 1) nlmeans_v3_kernel(const __grid_con
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     __syncwarp();
-    if (TMEM && warp == 0)
+    if (warp == 0)
     {
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" :: "r"(smem_u32(tmem_base_slot)) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
-    if (TMEM) asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
-    if (TMEM) asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     if (tid == 0)
     {
         mbar_expect_tx(bar, L::kTileBytes * (PRE ? 2 : 1));
@@ -507,27 +484,11 @@ __global__ void __launch_bounds__(NW * 32, 1) nlmeans_v3_kernel(const __grid_con
     const int seg_y0 = warp * RS;
     int rows = p.h - (Y0 + seg_y0);                                     // rows of this warp's strip inside the plane
     rows = rows < 0 ? 0 : (rows > RS ? RS : rows);
-    V3Acc<TMEM> acc;
-    if constexpr (TMEM)
-    {
-        const uint32_t base = *tmem_base_slot;
-        acc.taddr = base + ((uint32_t)(warp & 3) << 21) + (uint32_t)((warp >> 2) * RS * 8);   // lane 32 * (warp % 4) in bits 31..16
-        uint32_t z[8] = { 0, 0, 0, 0, 0, 0, 0, 0 };
-        for (int r = 0; r < RS; r++) acc.store(r, z);
-        acc.wait_store();
-    }
-    else
-    {
-        float *acc_ws = reinterpret_cast<float *>(smem + L::kOffWs);
-        float *acc_ps = reinterpret_cast<float *>(smem + L::kOffPs);
-        for (int i = tid; i < L::kTH * kTileW; i += kThreads)
-        {
-            acc_ws[i] = 0.f;
-            acc_ps[i] = 0.f;
-        }
-        acc.ws = acc_ws + seg_y0 * kTileW + lane * 4;
-        acc.ps = acc_ps + seg_y0 * kTileW + lane * 4;
-    }
+    V3Acc acc;
+    acc.taddr = *tmem_base_slot + ((uint32_t)(warp & 3) << 21) + (uint32_t)((warp >> 2) * RS * 8);   // lane 32 * (warp % 4) in bits 31..16
+    uint32_t z[8] = { 0, 0, 0, 0, 0, 0, 0, 0 };
+    for (int r = 0; r < RS; r++) acc.store(r, z);
+    acc.wait_store();
     mbar_wait(bar, 0);
     __syncthreads();
 
@@ -613,22 +574,21 @@ __global__ void __launch_bounds__(NW * 32, 1) nlmeans_v3_kernel(const __grid_con
                 if (X0 + x + i < p.w) drow[i] = o[i];
         }
     }
-    if (TMEM)
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    if (warp == 0)
     {
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncthreads();
-        if (warp == 0)
-        {
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" :: "r"(*tmem_base_slot) : "memory");
-        }
+        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" :: "r"(*tmem_base_slot) : "memory");
     }
 }
 
 
 // ---------------------------------------------------------------------------------------------------------------------
-// 16-bit samples (yuv420p10 planes; every sample <= kFast16Max = 1023, checked by the border kernel -- see
-// nlmeans_fast16_kernel for the contract and the integer stand-in that takes over otherwise).
+// 16-bit samples (yuv420p10 planes; every sample <= kMax10Bit = 1023).  A 16-bit container can hold samples above
+// 1023.  The border kernel raises a sticky flag when it sees one; this kernel then returns at once and the integer
+// kernel launched right behind it (which returns at once when the flag is clear) does the frame: same output either
+// way, no host round trip.
 //
 // Same march as the 8-bit group: a lane owns 4 adjacent pixels and walks down its strip with the vertical running sum V
 // of horizontal patch-row sums in registers.  The squared differences have no packed-integer instruction at this width;
@@ -837,12 +797,12 @@ __device__ __forceinline__ void v3_group16(const uint32_t *__restrict__ cur, con
     g.run(rows);
 }
 
-template <int NH, int NW, int RS, bool TMEM, int NBUF>
+template <int NH, int NW, int RS, int NBUF>
 __global__ void __launch_bounds__(NW * 32, 1) nlmeans_v3w_kernel(const __grid_constant__ FusedParams fp)
 {
     if (*fp.range_flag != 0u) return;               // samples above 10 bit seen: the integer kernel takes over
     constexpr int kThreads = NW * 32;
-    using L = V3Layout<NW, RS, TMEM, NBUF, 2>;
+    using L = V3Layout<NW, RS, NBUF, 2>;
     int pl = 0;
     while (pl + 1 < fp.nplanes && (int)blockIdx.x >= fp.first_tile[pl + 1]) pl++;
     const KernelParams &p = fp.k[pl];
@@ -864,14 +824,14 @@ __global__ void __launch_bounds__(NW * 32, 1) nlmeans_v3w_kernel(const __grid_co
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     __syncwarp();
-    if (TMEM && warp == 0)
+    if (warp == 0)
     {
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" :: "r"(smem_u32(tmem_base_slot)) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
-    if (TMEM) asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
-    if (TMEM) asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     if (tid == 0)
     {
         mbar_expect_tx(bar, L::kTileBytes);
@@ -892,27 +852,11 @@ __global__ void __launch_bounds__(NW * 32, 1) nlmeans_v3w_kernel(const __grid_co
     const int seg_y0 = warp * RS;
     int rows = p.h - (Y0 + seg_y0);
     rows = rows < 0 ? 0 : (rows > RS ? RS : rows);
-    V3Acc<TMEM> acc;
-    if constexpr (TMEM)
-    {
-        const uint32_t base = *tmem_base_slot;
-        acc.taddr = base + ((uint32_t)(warp & 3) << 21) + (uint32_t)((warp >> 2) * RS * 8);
-        uint32_t z[8] = { 0, 0, 0, 0, 0, 0, 0, 0 };
-        for (int r = 0; r < RS; r++) acc.store(r, z);
-        acc.wait_store();
-    }
-    else
-    {
-        float *acc_ws = reinterpret_cast<float *>(smem + L::kOffWs);
-        float *acc_ps = reinterpret_cast<float *>(smem + L::kOffPs);
-        for (int i = tid; i < L::kTH * kTileW; i += kThreads)
-        {
-            acc_ws[i] = 0.f;
-            acc_ps[i] = 0.f;
-        }
-        acc.ws = acc_ws + seg_y0 * kTileW + lane * 4;
-        acc.ps = acc_ps + seg_y0 * kTileW + lane * 4;
-    }
+    V3Acc acc;
+    acc.taddr = *tmem_base_slot + ((uint32_t)(warp & 3) << 21) + (uint32_t)((warp >> 2) * RS * 8);
+    uint32_t z[8] = { 0, 0, 0, 0, 0, 0, 0, 0 };
+    for (int r = 0; r < RS; r++) acc.store(r, z);
+    acc.wait_store();
     mbar_wait(bar, 0);
     __syncthreads();
 
@@ -985,14 +929,11 @@ __global__ void __launch_bounds__(NW * 32, 1) nlmeans_v3w_kernel(const __grid_co
                 if (X0 + x + i < p.w) drow[i] = o[i];
         }
     }
-    if (TMEM)
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    if (warp == 0)
     {
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncthreads();
-        if (warp == 0)
-        {
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" :: "r"(*tmem_base_slot) : "memory");
-        }
+        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" :: "r"(*tmem_base_slot) : "memory");
     }
 }

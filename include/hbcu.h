@@ -190,9 +190,11 @@ int  hbcu_nlmeans_filter_frame(hbcu_nlmeans_t *h, int64_t index, int navail, hbc
 /* orders a caller-owned CUDA stream (passed as void*) after all work queued on the handle so far */
 int  hbcu_nlmeans_stream_wait(hbcu_nlmeans_t *h, void *cuda_stream);
 int  hbcu_nlmeans_sync(hbcu_nlmeans_t *h);
-/* implementation selector for tests: 0 = auto (tiled sm_100a kernel when the
- * parameters fit, generic otherwise), 1 = force generic, 2 = force tiled,
- * 3 = tiled but integer-arithmetic variant (the one 16-bit planes use) */
+/* implementation selector for tests: 0 = auto (per plane: the v3 tile kernels
+ * where their conditions hold, else the integer tiled kernel where the patch
+ * and range fit its halo, else the generic kernel), 1 = force generic,
+ * 2 = as 0 but fail where 0 would take the generic kernel, 3 = integer tiled
+ * kernel where it fits, generic otherwise (the one >10-bit planes use) */
 int  hbcu_nlmeans_set_impl(hbcu_nlmeans_t *h, int impl);
 
 /* CUDA-event timing on the handle's compute stream (bench.py):

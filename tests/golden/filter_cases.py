@@ -69,6 +69,10 @@ def cases():
         w, h = 128, 80
         clip = synth.progressive_clip(FMT[depth], w, h, 4, seed=21)
         add(f"nlmeans_prefilter_median_reduce_{depth}", "hb_filter_nlmeans", "hb_filter_nlmeans_cuda", "y-strength=6:y-prefilter=514:threads=1", depth, w, h, clip)
+        # range 1 (no spatial displacement, only the temporal ones): chroma inherits it, so all three planes run it
+        add(f"nlmeans_range1_{depth}", "hb_filter_nlmeans", "hb_filter_nlmeans_cuda", "y-strength=6:y-range=1:y-frame-count=3", depth, w, h, clip)
+        if depth == 8:
+            add("nlmeans_range1_luma_8", "hb_filter_nlmeans", "hb_filter_nlmeans_cuda", "y-strength=6:y-range=1:y-frame-count=3:cb-strength=0", depth, w, h, clip)
 
         w, h = 160, 96
         clip, flags = synth.telecined_clip(FMT[depth], w, h, 16, seed=71)

@@ -91,7 +91,7 @@ def test_prefilter_modes(ref, cuda_filters, mode, fmt):
 
 @pytest.mark.parametrize("impl", ["1", "3"])
 def test_other_kernels_agree(ref, cuda_filters, monkeypatch, impl):
-    """generic (1) and integer-tiled (3) kernels on the same 8-bit clip the fast kernel handles by default"""
+    """generic (1) and integer-tiled (3) kernels on the same 8-bit clip the v3 kernel handles by default"""
     monkeypatch.setenv("HBCU_NLMEANS_IMPL", impl)
     w, h = 300, 150
     clip = synth.progressive_clip(FMT8, w, h, 4, seed=21)
@@ -124,28 +124,25 @@ def test_golden_digests(cuda_filters):
         assert [hashlib.sha256(f.tobytes()).hexdigest() for f in g.frames] == c["sha256"], name
 
 
-@pytest.mark.parametrize("ssd", ["0", "1"])
-def test_both_ssd_formulations(ref, cuda_filters, monkeypatch, ssd):
-    """fp32-prefix-sum (0) and VABSDIFF4+IDP4A (1) patch-row sums, patch sizes 3/5/7/9 over the three planes"""
-    monkeypatch.setenv("HBCU_NLMEANS_SSD", ssd)
+@pytest.mark.parametrize("s", ["y-strength=6:y-patch-size=7:cb-strength=5:cb-patch-size=5:cb-range=5:cr-patch-size=3",
+                               "y-strength=8:y-patch-size=9:y-range=5:y-frame-count=3"])
+def test_patch_sizes_3_5_7_9(ref, cuda_filters, s):
+    """patch sizes 3/5/7/9 over the three planes: per-plane launches where the patch sizes differ, the 8-warp shape of
+    patch 9"""
     w, h = 300, 170
     clip = synth.progressive_clip(FMT8, w, h, 4, seed=23)
-    for s in ("y-strength=6:y-patch-size=7:cb-strength=5:cb-patch-size=5:cb-range=5:cr-patch-size=3",
-              "y-strength=8:y-patch-size=9:y-range=5:y-frame-count=3"):
-        r, g = run_both(ref, cuda_filters, s, clip, FMT8, w, h)
-        assert_same(r, g)
+    r, g = run_both(ref, cuda_filters, s, clip, FMT8, w, h)
+    assert_same(r, g)
 
 
+@pytest.mark.parametrize("s", ["y-strength=6", "y-strength=10:y-patch-size=5:y-range=5:y-frame-count=3"])
 @pytest.mark.parametrize("fmt", [FMT8, FMT10])
-def test_round1_kernels_still_agree(ref, cuda_filters, monkeypatch, fmt):
-    """HBCU_NLMEANS_V3=off selects the round-1 fused kernels (nlmeans_fast8 / fast16), the baseline of the v3 levers in
-    profiles/r02b_v3_shape_sweep.txt: they stay bit-exact"""
-    monkeypatch.setenv("HBCU_NLMEANS_V3", "off")
+def test_ragged_clip_8_and_10bit(ref, cuda_filters, fmt, s):
+    """a 330 x 210 clip (ragged against every tile shape) in 8 and 10 bit, default kernels"""
     w, h = 330, 210
     clip = synth.progressive_clip(fmt, w, h, 4, seed=33)
-    for s in ("y-strength=6", "y-strength=10:y-patch-size=5:y-range=5:y-frame-count=3"):
-        r, g = run_both(ref, cuda_filters, s, clip, fmt, w, h)
-        assert_same(r, g)
+    r, g = run_both(ref, cuda_filters, s, clip, fmt, w, h)
+    assert_same(r, g)
 
 
 def clip10_extreme(w, h, seed=9):
@@ -159,8 +156,9 @@ def clip10_extreme(w, h, seed=9):
 
 @pytest.mark.parametrize("impl", ["0", "3", "1"])
 def test_10bit_kernels_agree(ref, cuda_filters, monkeypatch, impl):
-    """fast fp32-exact 10-bit kernel (0), integer tiled kernel (3), generic kernel (1): patch 7/5/3, ranges 3/5/7,
-    every alignment of the compare window (dx0 mod 4), 3-frame window, ragged size"""
+    """default 10-bit kernel (0), integer tiled kernel (3), generic kernel (1): patch 7/5/3, ranges 3/5/7, every alignment
+    of the compare window (dx0 mod 4), 3-frame window, ragged size; the second setting gives luma and chroma different
+    patch sizes, so by default each plane runs its own launch"""
     monkeypatch.setenv("HBCU_NLMEANS_IMPL", impl)
     w, h = 330, 210
     clip = synth.progressive_clip(FMT10, w, h, 4, seed=31)
@@ -179,7 +177,7 @@ def test_10bit_extreme_content(ref, cuda_filters):
 
 def test_10bit_container_with_out_of_range_samples(ref, cuda_filters):
     """a yuv420p10 stream whose 16-bit words exceed 1023 from the third frame on: the border kernel raises the range
-    flag, the fast kernel stands down and the integer kernel produces the frames -- still the reference's output"""
+    flag, the v3 kernel stands down and the integer kernel produces the frames -- still the reference's output"""
     w, h = 256, 128
     clip = synth.progressive_clip(FMT10, w, h, 5, seed=33).copy()
     v = clip.view(np.uint16).reshape(5, -1)
